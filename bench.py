@@ -52,7 +52,15 @@ def parse():
     ap.add_argument('--no-fused', action='store_true',
                     help='materialise pre-offsets / offset / mask (reference operator boundaries) instead of the '
                          'fused DynAgg gather')
-    return ap.parse_args()
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='after the timed steps, write the outputs of the last one as DIR/<name>.npy (rank 0; below 64 MB '
+                         'in all: a larger output is sampled at fixed seeded positions)')
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and args.impl != 'ours':
+        ap.error('--dump-outputs writes the outputs of the GPU path (--impl ours)')
+    return args
 
 
 # ----------------------------------------------------------------------------------------------------------
@@ -129,6 +137,28 @@ def hot_path_step(M, d, b, r, match_mode, dcn_mode, fused=True):
         f = M.mrapa_attention(d[f'emb_t{c}'], d[f'emb{c}'], d[f'ass{c}'], r)
         outs += [y, f]
     return outs
+
+
+OUTPUT_NAMES = ('match_index', 'match_similarity', 'dcn_relu3_1', 'fusion_relu3_1', 'dcn_relu2_1', 'fusion_relu2_1',
+                'dcn_relu1_1', 'fusion_relu1_1')   # hot_path_step's outputs, in order
+DUMP_BYTES = 60 << 20           # all the .npy files together stay below 64 MB
+
+
+def dump_outputs(outs, out_dir):
+    """Write hot_path_step's outputs as out_dir/<name>.npy: floating outputs as float32, integer ones as float64 (exact).
+    An output larger than its share of DUMP_BYTES is stored as the values at a sorted sample of flat (logical NCHW)
+    positions drawn from a generator seeded by the output's place in the list, so that two runs with the same
+    arguments, on any build, store the same elements."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    share = DUMP_BYTES // len(outs)
+    for k, (name, t) in enumerate(zip(OUTPUT_NAMES, outs, strict=True)):
+        dt = torch.float32 if t.is_floating_point() else torch.float64
+        n = share // dt.itemsize
+        if t.numel() > n:
+            pos = torch.randint(t.numel(), (n,), generator=torch.Generator().manual_seed(k)).sort().values
+            t = t.flatten()[pos.to(t.device)]
+        np.save(os.path.join(out_dir, name + '.npy'), t.detach().to(dt).cpu().contiguous().numpy())
 
 
 # ----------------------------------------------------------------------------------------------------------
@@ -272,7 +302,7 @@ def run_reference(args):
     n_img = 2
     for _ in range(max(1, min(args.warmup, 1))):
         cpu_hot_path(n_img, args.refs)
-    steps = max(1, min(args.steps, 5))
+    steps = args.steps
     # the timed region is the hot path itself (cpu_hot_path's own clock), as in the GPU arm, whose inputs also
     # exist before the clock starts: drawing the synthetic tensors (0.4 GB of randn per image) is not part of it
     dt = sum(cpu_hot_path(n_img, args.refs)['total_s'] for _ in range(steps))
@@ -412,8 +442,9 @@ def main():
     ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     barrier()
     ev0.record()
-    for _ in range(args.steps):
+    for _ in range(args.steps - 1):
         hot_path_step(M, d, b, r, args.match_mode, args.dcn_mode, fused)
+    outs = hot_path_step(M, d, b, r, args.match_mode, args.dcn_mode, fused)
     ev1.record()
     barrier()
     ms = ev0.elapsed_time(ev1)
@@ -426,6 +457,9 @@ def main():
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
     ms_max = float(t.item())
     value = b * world * args.steps / (ms_max / 1e3)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(outs, args.dump_outputs)
+    del outs
 
     # ---- sustained: the same step back to back for >= 3 s (the timed region above is a fraction of a second)
     extras = {}

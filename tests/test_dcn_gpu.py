@@ -1,5 +1,6 @@
-"""Parity of the CUDA DCNv2 (through the C ABI) against the oracle, the golden vectors generated from the
-reference's DynAgg, and -- when oracle/_ref holds the reference's own CUDA extension -- the reference kernels."""
+"""Parity of the CUDA DCNv2 (through the C ABI and the torch extension module) against the oracle, the golden vectors
+generated from the reference's DynAgg, and -- when oracle/_ref holds the reference's own CUDA extension -- the
+reference kernels."""
 import os
 
 import pytest
@@ -349,73 +350,97 @@ _REF_SO = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__)
                        'deform_conv_ext_ref.so')
 
 
-@pytest.mark.skipif(not os.path.exists(_REF_SO), reason='reference CUDA extension not prebuilt (oracle/build.py --ref)')
-def test_against_reference_cuda_extension():
-    """The reference's own deform_conv_ext, compiled unmodified for sm_100a into oracle/_ref/ (checker only)."""
+def _reference_ext():
+    """The reference's own deform_conv_ext, compiled unmodified for sm_100a into oracle/_ref/ by `oracle/build.py --ref`
+    where the reference's sources are at hand (checker only), or None."""
+    if not os.path.exists(_REF_SO):
+        return None
     import importlib.util
     spec = importlib.util.spec_from_file_location('deform_conv_ext_ref', _REF_SO)
     ext = importlib.util.module_from_spec(spec)
     spec.loader.exec_module(ext)
-    x, off, mask, wgt, bias = (t.to(DEV) for t in _rand_problem(2, 64, 24, 20, 64, 8, 31, off_scale=4.0))
-    out_ref = x.new_empty(2, 64, 24, 20)
-    ext.modulated_deform_conv_forward(x, wgt, bias, x.new_empty(0), off, mask, out_ref, x.new_empty(0), 3, 3, 1, 1, 1, 1,
-                                      1, 1, 1, 8, True)
-    out = D.dcn_forward_raw(x, off, mask, wgt, bias, (1, 1), (1, 1), (1, 1), 1, 8)
-    assert rel_err(out, out_ref) <= TOL
-    # backward through the reference's own kernels
-    go = torch.randn_like(out_ref)
-    gr = [torch.zeros_like(t) for t in (x, wgt, bias, off, mask)]
-    ext.modulated_deform_conv_backward(x, wgt, bias, x.new_empty(0), off, mask, x.new_empty(0), gr[0], gr[1], gr[2],
-                                       gr[3], gr[4], go, 3, 3, 1, 1, 1, 1, 1, 1, 1, 8, True)
-    gi, goff, gm, gw, gb = D.dcn_backward_raw(x, off, mask, wgt, go, (1, 1), (1, 1), (1, 1), 1, 8, True)
-    for got, ref, name in ((gi, gr[0], 'input'), (gw, gr[1], 'weight'), (gb, gr[2], 'bias'), (goff, gr[3], 'offset'),
-                           (gm, gr[4], 'mask')):
-        assert rel_err(got, ref) <= TOL, name
-    # DCNv1 forward of the reference extension
-    out1 = x.new_empty(2, 64, 24, 20)
-    ext.deform_conv_forward(x, wgt, off, out1, x.new_empty(0), x.new_empty(0), 3, 3, 1, 1, 1, 1, 1, 1, 1, 8, 2)
-    mine = M.deform_conv(x, off, wgt, 1, 1, 1, 1, 8)
-    assert rel_err(mine, out1) <= TOL
+    return ext
+
+
+def _oracle_dcn(x, off, mask, wgt, bias, go, dg=8):
+    """fp64 oracle of a 3x3 / stride 1 / pad 1 DCN on CPU tensors: DCNv2 output, its five gradients for grad_output
+    `go`, and the DCNv1 output (mask 1, no bias)."""
+    f64 = torch.float64
+    want = {'output': oracle.modulated_deform_conv_oracle(x, off, mask, wgt, bias, 1, 1, 1, 1, dg, dtype=f64)}
+    grads = oracle.modulated_deform_conv_backward_oracle(x, off, mask, wgt, bias, go, 1, 1, 1, 1, dg, dtype=f64)
+    want.update(zip(('input', 'offset', 'mask', 'weight', 'bias'), grads))
+    want['dcnv1'] = oracle.modulated_deform_conv_oracle(x, off, torch.ones_like(mask), wgt, None, 1, 1, 1, 1, dg, dtype=f64)
+    return want
+
+
+def _drive_ext(ext, x, off, mask, wgt, bias, go, grad_weight_init=0.0, grad_bias_init=0.0):
+    """Call a deform_conv_ext module the way basicsr/ops/dcn/deform_conv.py:147-170 does (caller-allocated output, size-0
+    `ones` / `columns` scratch, zero-initialised input / offset / mask gradients; grad_weight / grad_bias start at the
+    given values).  Returns the results keyed like _oracle_dcn, and deform_conv_forward's return value."""
+    empty = x.new_empty(0)
+    got = {'output': x.new_empty(x.shape[0], wgt.shape[0], *x.shape[2:])}   # 3x3, stride 1, pad 1
+    ext.modulated_deform_conv_forward(x, wgt, bias, empty, off, mask, got['output'], empty, 3, 3, 1, 1, 1, 1, 1, 1, 1, 8,
+                                      True)
+    g = [torch.zeros_like(t) for t in (x, wgt, bias, off, mask)]
+    g[1].fill_(grad_weight_init)
+    g[2].fill_(grad_bias_init)
+    ext.modulated_deform_conv_backward(x, wgt, bias, empty, off, mask, empty, g[0], g[1], g[2], g[3], g[4], go, 3, 3, 1,
+                                       1, 1, 1, 1, 1, 1, 8, True)
+    got.update(zip(('input', 'weight', 'bias', 'offset', 'mask'), g))
+    got['dcnv1'] = torch.empty_like(got['output'])
+    rc = ext.deform_conv_forward(x, wgt, off, got['dcnv1'], empty, empty, 3, 3, 1, 1, 1, 1, 1, 1, 1, 8, 2)
+    return got, rc
+
+
+def test_against_reference_cuda_extension():
+    """The product DCN (dcn_forward_raw, dcn_backward_raw, deform_conv) on a problem with many samples at and beyond the
+    image border (offsets ~ N(0, 4^2)): against the fp64 oracle, and, where oracle/_ref holds the reference's own
+    deform_conv_ext, against the reference's kernels on the same inputs."""
+    cpu = _rand_problem(2, 64, 24, 20, 64, 8, 31, off_scale=4.0)
+    go = torch.randn(2, 64, 24, 20, generator=torch.Generator().manual_seed(3))
+    want = _oracle_dcn(*cpu, go)
+    x, off, mask, wgt, bias, go = (t.to(DEV) for t in cpu + (go,))
+    got = {'output': D.dcn_forward_raw(x, off, mask, wgt, bias, (1, 1), (1, 1), (1, 1), 1, 8)}
+    got.update(zip(('input', 'offset', 'mask', 'weight', 'bias'),
+                   D.dcn_backward_raw(x, off, mask, wgt, go, (1, 1), (1, 1), (1, 1), 1, 8, True)))
+    got['dcnv1'] = M.deform_conv(x, off, wgt, 1, 1, 1, 1, 8)
+    for name in want:
+        assert rel_err(got[name], want[name]) <= TOL, name
+    ref = _reference_ext()
+    if ref is not None:
+        ref_got, _ = _drive_ext(ref, x, off, mask, wgt, bias, go)
+        for name in ref_got:
+            assert rel_err(got[name], ref_got[name]) <= TOL, ('reference extension', name)
 
 
 def test_torch_extension_module_is_call_compatible_with_the_reference_extension():
     """mrefsr_b200/torch_ext/deform_conv_ext.so -- the pybind module that replaces the reference's deform_conv_ext build
-    (csrc/torch_ext/deform_conv_ext.cpp) -- and the reference's own extension (oracle/_ref, checker) are driven with the
-    SAME argument lists, the way basicsr/ops/dcn/deform_conv.py:147-170 calls them: caller-allocated output, size-0
-    `ones` / `columns` scratch, zero-initialised gradients, grad_weight / grad_bias accumulated."""
-    import importlib.util
+    (csrc/torch_ext/deform_conv_ext.cpp) -- driven with the reference's argument lists, grad_weight / grad_bias
+    accumulated into (deform_conv_cuda.cpp:571-685): against the fp64 oracle, and, where oracle/_ref holds the
+    reference's own deform_conv_ext, against the reference driven with the same calls."""
     from mrefsr_b200 import build as B
     ours = B.load_torch_ext()
-    spec = importlib.util.spec_from_file_location('deform_conv_ext_ref', _REF_SO)
-    ref = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(ref)
-    x, off, mask, wgt, bias = (t.to(DEV) for t in _rand_problem(2, 64, 24, 20, 64, 8, 33, off_scale=3.0))
-    empty = x.new_empty(0)
-    outs, grads = {}, {}
-    go = torch.randn(2, 64, 24, 20, generator=torch.Generator().manual_seed(2)).to(DEV)
-    for name, ext in (('ours', ours), ('ref', ref)):
-        out = x.new_empty(2, 64, 24, 20)
-        ext.modulated_deform_conv_forward(x, wgt, bias, empty, off, mask, out, empty, 3, 3, 1, 1, 1, 1, 1, 1, 1, 8, True)
-        outs[name] = out
-        g = [torch.zeros_like(t) for t in (x, wgt, bias, off, mask)]
-        g[1].fill_(0.5)                                        # pre-existing content: grad_weight / grad_bias accumulate
-        g[2].fill_(-1.0)
-        ext.modulated_deform_conv_backward(x, wgt, bias, empty, off, mask, empty, g[0], g[1], g[2], g[3], g[4], go, 3, 3,
-                                           1, 1, 1, 1, 1, 1, 1, 8, True)
-        grads[name] = g
-    assert rel_err(outs['ours'], outs['ref']) <= TOL
-    for a, b, name in zip(grads['ours'], grads['ref'], ('input', 'weight', 'bias', 'offset', 'mask')):
-        assert rel_err(a, b) <= TOL, name
-    # DCNv1 export, the reference's (W, H) argument order; int return value 1
-    o1, o2 = x.new_empty(2, 64, 24, 20), x.new_empty(2, 64, 24, 20)
-    assert ours.deform_conv_forward(x, wgt, off, o1, empty, empty, 3, 3, 1, 1, 1, 1, 1, 1, 1, 8, 2) == 1
-    ref.deform_conv_forward(x, wgt, off, o2, empty, empty, 3, 3, 1, 1, 1, 1, 1, 1, 1, 8, 2)
-    assert rel_err(o1, o2) <= TOL
+    cpu = _rand_problem(2, 64, 24, 20, 64, 8, 33, off_scale=3.0)
+    go = torch.randn(2, 64, 24, 20, generator=torch.Generator().manual_seed(2))
+    want = _oracle_dcn(*cpu, go)
+    want['weight'] = want['weight'] + 0.5                    # pre-existing content: grad_weight / grad_bias accumulate
+    want['bias'] = want['bias'] - 1.0
+    x, off, mask, wgt, bias, go = (t.to(DEV) for t in cpu + (go,))
+    got, rc = _drive_ext(ours, x, off, mask, wgt, bias, go, 0.5, -1.0)
+    assert rc == 1                                           # DCNv1 export: the reference's int return value
+    for name in want:
+        assert rel_err(got[name], want[name]) <= TOL, name
+    ref = _reference_ext()
+    if ref is not None:
+        ref_got, _ = _drive_ext(ref, x, off, mask, wgt, bias, go, 0.5, -1.0)
+        for name in ref_got:
+            assert rel_err(got[name], ref_got[name]) <= TOL, ('reference extension', name)
     # fp16 tensors are accepted like the reference's AT_DISPATCH_FLOATING_TYPES_AND_HALF (computed in fp32 here)
+    empty = x.new_empty(0)
     oh = x.new_empty(2, 64, 24, 20).half()
     ours.modulated_deform_conv_forward(x.half(), wgt.half(), bias.half(), empty, off.half(), mask.half(), oh, empty, 3, 3,
                                        1, 1, 1, 1, 1, 1, 1, 8, True)
-    assert rel_err(oh.float(), outs['ref']) <= 2e-2
+    assert rel_err(oh.float(), want['output']) <= 2e-2
     # the reference's error behaviour: kernel-shape mismatch -> RuntimeError
     with pytest.raises(RuntimeError, match="kernel shape won't match"):
         ours.modulated_deform_conv_forward(x, wgt, bias, empty, off, mask, x.new_empty(2, 64, 24, 20), empty, 5, 5, 1, 1, 1,
