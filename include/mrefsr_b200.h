@@ -123,15 +123,6 @@ MREFSR_API size_t mrefsr_dcn_workspace_bytes(int B, int C, int H, int W, int Co,
  * consecutive positions (0), patch width, patch height, number of tiles}; coords (optional, 3 ints per row, room for
  * max_rows rows) receives (sample, oy, ox) of every row of every tile, (-1, -1, -1) for padding rows. */
 MREFSR_API int mrefsr_dcn_tile_plan(int B, int Ho, int Wo, int* meta, int* coords, size_t max_rows);
-/* Same for the shared-memory window kernel (csrc/dcn_win.cu; 3x3, stride 1, pad 1 calls: every DCN call of MRefSR,
- * ref_mrapa_restoration_arch.py:74-76): meta[10] = {served (0: the call falls back to the 256-row kernel), tiles of
- * 128 rows, patch width, patch height, patches per tile, window width, window height, margin, pipeline stages, dynamic
- * shared memory bytes}; coords as above with 128 rows per tile. */
-/* Opt-in switch of that kernel (process-wide; also env MREFSR_DCN_WIN=1 at first use).  Returns the previous setting.
- * Same results bit for bit either way; see DESIGN.md section 2.2b for when it pays. */
-MREFSR_API int mrefsr_dcn_window_enable(int on);
-MREFSR_API int mrefsr_dcn_win_plan(int B, int C, int H, int W, int Co, int deformable_group, int* meta, int* coords,
-                                   size_t max_rows);
 MREFSR_API int mrefsr_modulated_deform_conv_forward(const float* input, const float* weight, const float* bias,
                                          const float* offset, const float* mask, float* output, int B, int C, int H,
                                          int W, int Co, int kh, int kw, int stride_h, int stride_w, int pad_h,

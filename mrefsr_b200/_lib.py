@@ -27,8 +27,6 @@ SIGNATURES = {
     'mrefsr_pre_offsets': (c_int, [_P, _I, _I, _I, _P, _P, _P, _P]),
     'mrefsr_dcn_workspace_bytes': (c_size_t, [_I] * 17),
     'mrefsr_dcn_tile_plan': (c_int, [_I, _I, _I, _P, _P, c_size_t]),
-    'mrefsr_dcn_window_enable': (c_int, [_I]),
-    'mrefsr_dcn_win_plan': (c_int, [_I, _I, _I, _I, _I, _I, _P, _P, c_size_t]),
     'mrefsr_modulated_deform_conv_forward': (c_int, [_P] * 6 + [_I] * 17 + [_P, c_size_t, _P]),
     'mrefsr_modulated_deform_conv_backward': (c_int, [_P] * 10 + [_I] * 17 + [_P, c_size_t, _P]),
     'mrefsr_gemm_tf32_nt': (c_int, [_P, _I, ctypes.c_longlong, _P, _I, ctypes.c_longlong, _P, _I, ctypes.c_longlong,

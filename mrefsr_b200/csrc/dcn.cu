@@ -700,16 +700,6 @@ static int bwd_chunk(const DcnShape& s) {
     return (int)nb;
 }
 
-// MREFSR_DCN_BWD_MERGE=0 (tuning knob / cross-check; default 1): separate coordinate-gradient and column kernels
-static bool bwd_merge_enabled() {
-    static int on = -1;
-    if (on < 0) {
-        const char* e = getenv("MREFSR_DCN_BWD_MERGE");
-        on = (e && e[0] == '0') ? 0 : 1;
-    }
-    return on == 1;
-}
-
 static int grid_for(size_t total) {
     size_t blocks = (total + 255) / 256;
     const size_t cap = (size_t)sm_count() * 32;
@@ -737,16 +727,6 @@ int mrefsr_dcn_tile_plan(int B, int Ho, int Wo, int* meta, int* coords, size_t m
     MREFSR_CHECK(B > 0 && Ho > 0 && Wo > 0 && meta, ERR_BAD_ARG, "tile plan: bad arguments");
     MREFSR_CHECK((long long)B * Ho * Wo < (1ll << 31) - 256, ERR_BAD_ARG, "tile plan: too many positions");
     return dcn_tc_tile_plan(B, Ho, Wo, meta, coords, max_rows);
-}
-
-int mrefsr_dcn_window_enable(int on) { return dcn_win_set_mode(on); }
-
-int mrefsr_dcn_win_plan(int B, int C, int H, int W, int Co, int deformable_group, int* meta, int* coords,
-                        size_t max_rows) {
-    MREFSR_CHECK(B > 0 && C > 0 && H > 0 && W > 0 && Co > 0 && deformable_group > 0 && meta, ERR_BAD_ARG,
-                 "window plan: bad arguments");
-    MREFSR_CHECK((long long)B * H * W < (1ll << 31) - 256, ERR_BAD_ARG, "window plan: too many positions");
-    return dcn_win_plan_query(B, C, H, W, Co, deformable_group, meta, coords, max_rows);
 }
 
 size_t mrefsr_dcn_workspace_bytes(int B, int C, int H, int W, int Co, int kh, int kw, int stride_h, int stride_w,
@@ -865,7 +845,7 @@ int mrefsr_modulated_deform_conv_backward(const float* input, const float* weigh
             count_launches(1);
         }
         // coordinate gradients and recomputed columns from ONE gather when the backward wants both
-        const bool merged = grad_offset && nhwc_coord && tc_gw && bwd_merge_enabled();
+        const bool merged = grad_offset && nhwc_coord && tc_gw;
         if (merged) {
             dcn_bwd_coord_cols_kernel<<<grid_for((size_t)nb * deformable_group * P), 256, 0, st>>>(
                 xt, offset, mask, gcol, grad_offset, grad_mask, col, s, b0, nb);

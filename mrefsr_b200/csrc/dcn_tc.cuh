@@ -1,5 +1,5 @@
-// mrefsr_b200/csrc/dcn_tc.cuh -- definitions shared by the tcgen05 DCN forward kernels (dcn_tc.cu: 256-row tiles,
-// corners gathered through L1; dcn_win.cu: 128-row tiles, corners gathered from TMA-staged shared-memory windows).
+// mrefsr_b200/csrc/dcn_tc.cuh -- the tcgen05 DCN forward's tile geometry, parameters and device helpers
+// (dcn_tc.cu); dcn.cu's backward shares the tf32 rounding.
 #pragma once
 #include "dcn_common.cuh"
 
@@ -8,14 +8,6 @@ namespace mrefsr {
 constexpr int TBM = 256;            // rows (output positions) per CTA tile
 constexpr int TBK = 32;             // fp32 channels per K step (128-byte rows)
 constexpr int T_A_BYTES = TBM * 128;
-constexpr int T_PW = 16;             // producer warps: sample table (T_AHEAD K steps ahead) + gather; warps 0..3 also drain TMEM
-constexpr int T_RSTEP = T_PW * 8;    // row stride between a thread's gather items (a warp covers 8 rows x 4 chunks)
-constexpr int T_ITEMS = TBM / T_RSTEP;             // gather items (row, 8-channel chunk) per thread per K step (2)
-constexpr int T_PRODUCERS = T_PW * 32;
-constexpr int T_MMA_WARP = T_PW;
-constexpr int T_THREADS = T_PRODUCERS + 32;        // + the MMA warp (17 warps: one sub-partition hosts 5 -> 96 registers/thread)
-constexpr int T_NTAB = 3;                          // sample-table ring depth
-constexpr int T_AHEAD = 1;                         // tables are decoded this many K steps before their gather
 constexpr int T_SMEM_BUDGET = 150 * 1024;          // stage ring; the rest of the 228 KB stays L1 for the gather
 
 struct DcnTcParams {
@@ -40,11 +32,7 @@ struct DcnTcParams {
     // positions (nsx patches per output row, nsub per sample), so that the bilinear corners of x- AND y-neighbours
     // fall into the same K step and hit in L1.
     int tile2d, tx_log, ty_log, sub_log, subs_log, nsx, nsub;
-    // dcn_win.cu only: per patch a (wx x wy)-pixel window of the NHWC input, mlo pixels of margin on the low side,
-    // is staged in shared memory; win_rows = 128-byte rows reserved per patch window (multiple of 8),
-    // win_bytes = bytes of one window buffer (all patches of a tile)
-    int wx, wy, mlo, win_rows, win_bytes, npatch, rdepth, dbg;
-    long long* trace;    // debug builds only (MREFSR_DCN_DEBUG)   // rdepth: raw offset / mask ring depth in K steps
+    int dbg;             // ablation bits, read by variant builds only (MREFSR_DCN_DEBUG)
 };
 
 // (tile, row within the tile) -> (sample, oy, ox); false for padding rows
@@ -109,11 +97,5 @@ __device__ __forceinline__ int ldg_early_s32(const int* p) {
     asm volatile("ld.global.nc.s32 %0, [%1];" : "=r"(v) : "l"(p));
     return v;
 }
-
-// dcn_win.cu: shared-memory window gather.  1: shape not served (caller falls back), 0: launched, < 0: error
-int dcn_win_launch(const CUtensorMap& mapW, const float* xt, const float* off, const float* mask,
-                   const long long* max_idx, const float* bias, DcnTcParams prm, cudaStream_t st);
-int dcn_win_set_mode(int on);
-int dcn_win_plan_query(int B, int C, int H, int W, int Co, int DG, int* meta, int* coords, size_t max_rows);
 
 }  // namespace mrefsr

@@ -61,36 +61,3 @@ def test_batches_by_shape_is_an_order_preserving_partition(keys, max_batch):
         sizes = [len(idxs) for kk, idxs in got if kk == k]
         assert all(s == max_batch for s in sizes[:-1])
 
-
-@settings(max_examples=60, deadline=None)
-@given(b=st.integers(1, 4), h=st.integers(3, 90), w=st.integers(3, 90), c=st.sampled_from([64, 128, 256]))
-def test_window_kernel_plan_covers_every_position_once_and_fits_shared_memory(b, h, w, c):
-    """Host logic of csrc/dcn_win.cu: when it serves a shape, its 128-row tiles of patches hit every output position
-    exactly once, a patch never straddles samples, the window is the patch plus 2 + 2 * margin pixels in each direction,
-    and the dynamic shared memory stays within the 227 KB a CTA may have."""
-    lib = _lib.lib()
-    meta = (ctypes.c_int * 10)()
-    assert lib.mrefsr_dcn_win_plan(b, c, h, w, c, 8, ctypes.cast(meta, ctypes.c_void_p), None, 0) == 0
-    served, tiles, pw, ph, npatch, wx, wy, margin, stages, smem = list(meta)
-    if not served:
-        return
-    assert pw * ph * npatch == 128 and (pw, ph) in ((16, 8), (8, 16), (8, 8))
-    assert wx == pw + 2 + 2 * margin and wy == ph + 2 + 2 * margin and margin in (2, 3) and 2 <= stages <= 4
-    assert smem <= 227 * 1024
-    assert tiles * 128 <= b * h * w * 1.4 + 128           # at most 40 % padding rows
-    coords = np.full((tiles * 128, 3), -7, dtype=np.int32)
-    assert lib.mrefsr_dcn_win_plan(b, c, h, w, c, 8, ctypes.cast(meta, ctypes.c_void_p), coords.ctypes.data_as(ctypes.c_void_p),
-                                   tiles * 128) == 0
-    valid = coords[:, 0] >= 0
-    assert (coords[~valid] == -1).all()
-    cc = coords[valid].astype(np.int64)
-    assert (cc[:, 0] < b).all() and (cc[:, 1] < h).all() and (cc[:, 2] < w).all() and (cc[:, 1:] >= 0).all()
-    lin = (cc[:, 0] * h + cc[:, 1]) * w + cc[:, 2]
-    assert len(lin) == b * h * w == len(np.unique(lin))
-    per = pw * ph
-    for k in range(0, len(coords), per):
-        blk = coords[k:k + per]
-        blk = blk[blk[:, 0] >= 0]
-        if len(blk):
-            assert (blk[:, 0] == blk[0, 0]).all()
-            assert blk[:, 1].max() - blk[:, 1].min() < ph and blk[:, 2].max() - blk[:, 2].min() < pw

@@ -1,9 +1,9 @@
 """A/B timing of the fused DynAgg + DCNv2 launches on bench.py's config-2 inputs, per scale.
 
-    MREFSR_LIB=<variant .so> MREFSR_DCN_TILE=linear|2d python tools/dcn_ab.py [tag]
+    MREFSR_LIB=<variant .so> python tools/dcn_ab.py [tag]
 
-Prints one JSON line per (flow kind, scale): per-launch device time of dcn_tc_kernel (CUDA events recorded inside
-the library).  Flow kinds: 'bench' = the arg-max maps of bench.py's synthetic references (3 translated, 2 independent
+Prints one JSON line per (flow kind, scale): per-launch device time of dcn_tc_split_kernel (CUDA events recorded
+inside the library).  Flow kinds: 'bench' = the arg-max maps of bench.py's synthetic references (3 translated, 2 independent
 per image), 'coherent' = every reference a translation, 'random' = uniformly random arg-max maps.
 """
 import json

@@ -1,5 +1,5 @@
-"""Ablation timing of the DCN window kernel (variant build with -DMREFSR_DCN_DEBUG; MREFSR_DCN_DBG bit mask, see
-csrc/dcn_win.cu).  Results are wrong by design; only the time matters.  One JSON line per scale."""
+"""Ablation timing of the DCN forward kernel (variant build with -DMREFSR_DCN_DEBUG; MREFSR_DCN_DBG bit mask, see
+csrc/dcn_tc.cu).  Results are wrong by design; only the time matters.  One JSON line per scale."""
 import json
 import os
 import sys
