@@ -31,25 +31,43 @@ def _pair(v):
     return (v, v) if isinstance(v, int) else tuple(v)
 
 
-def _columns(x, offset, mask, kh, kw, stride, padding, dilation, dg):
-    """Deformable im2col: [B, Cin, kh*kw, Ho*Wo] (value * mask)."""
-    b, cin, h, w = x.shape
+def sampling_positions(offset, kh, kw, stride, padding, dilation, dg, dtype, fp32_positions=False):
+    """Sampling positions (him, wim), each [B, dg, kh*kw, Ho, Wo], of offset [B, 2*dg*kh*kw, Ho, Wo]:
+    h_out*stride - pad + i*dil + offset (dy in channel 2*(g*K+k), dx in channel 2*(g*K+k)+1), in `dtype`.
+
+    fp32_positions: the positions take the value of the fp32 sum (h_out*stride - pad + i*dil) + offset, one rounding,
+    as the reference computes them (deform_conv_cuda_kernel.cu, modulated_deformable_im2col_gpu_kernel and
+    modulated_deformable_col2im_coord_gpu_kernel: `h_in + i * dilation_h + offset_h` in scalar_t) and as the kernels
+    of this package do.  Their derivative with respect to the offset stays 1 (straight-through).  The exact sum (the
+    default) differs where that rounding carries a point across an integer, and the offset gradient jumps there."""
     sh, sw = stride
     ph, pw = padding
     dh, dw = dilation
-    ho = (h + 2 * ph - (dh * (kh - 1) + 1)) // sh + 1
-    wo = (w + 2 * pw - (dw * (kw - 1) + 1)) // sw + 1
+    kk = kh * kw
+    b, _, ho, wo = offset.shape
+    off = offset.view(b, dg, kk, 2, ho, wo)
+    ys = (torch.arange(ho, dtype=dtype) * sh - ph).view(1, 1, 1, ho, 1)
+    xs = (torch.arange(wo, dtype=dtype) * sw - pw).view(1, 1, 1, 1, wo)
+    ki = (torch.arange(kk) // kw).to(dtype).view(1, 1, kk, 1, 1) * dh
+    kj = (torch.arange(kk) % kw).to(dtype).view(1, 1, kk, 1, 1) * dw
+    him = ys + ki + off[:, :, :, 0]
+    wim = xs + kj + off[:, :, :, 1]
+    if fp32_positions:
+        # |fp32 sum - exact sum| is one rounding of the sum, so the difference and the re-addition are exact in fp64
+        him = him + ((ys + ki).float() + off[:, :, :, 0].float() - him).detach()
+        wim = wim + ((xs + kj).float() + off[:, :, :, 1].float() - wim).detach()
+    return him, wim
+
+
+def _columns(x, offset, mask, kh, kw, stride, padding, dilation, dg, fp32_positions=False):
+    """Deformable im2col: [B, Cin, kh*kw, Ho*Wo] (value * mask).  fp32_positions: see sampling_positions."""
+    b, cin, h, w = x.shape
     kk = kh * kw
     cg = cin // dg
     dt = x.dtype
-    off = offset.view(b, dg, kk, 2, ho, wo)
+    ho, wo = offset.shape[2:]
     msk = mask.view(b, dg, kk, ho, wo)
-    ys = (torch.arange(ho, dtype=dt) * sh - ph).view(1, 1, 1, ho, 1)
-    xs = (torch.arange(wo, dtype=dt) * sw - pw).view(1, 1, 1, 1, wo)
-    ki = (torch.arange(kk) // kw).to(dt).view(1, 1, kk, 1, 1) * dh
-    kj = (torch.arange(kk) % kw).to(dt).view(1, 1, kk, 1, 1) * dw
-    him = ys + ki + off[:, :, :, 0]                         # [B, dg, kk, Ho, Wo]
-    wim = xs + kj + off[:, :, :, 1]
+    him, wim = sampling_positions(offset, kh, kw, stride, padding, dilation, dg, dt, fp32_positions)
     inside = (him > -1) & (wim > -1) & (him < h) & (wim < w)
     hl = torch.floor(him)
     wl = torch.floor(wim)
@@ -72,15 +90,15 @@ def _columns(x, offset, mask, kh, kw, stride, padding, dilation, dg):
 
 
 def modulated_deform_conv_oracle(x, offset, mask, weight, bias=None, stride=1, padding=0, dilation=1,
-                                 groups=1, deformable_groups=1, dtype=None):
+                                 groups=1, deformable_groups=1, dtype=None, fp32_positions=False):
     """out[B, Cout, Ho, Wo]; argument meaning as ModulatedDeformConvFunction.forward
-    (basicsr/ops/dcn/deform_conv.py:124-153)."""
+    (basicsr/ops/dcn/deform_conv.py:124-153).  fp32_positions: see sampling_positions."""
     dtype = dtype or x.dtype
     x, offset, mask, weight = (t.to(dtype) for t in (x, offset, mask, weight))
     stride, padding, dilation = _pair(stride), _pair(padding), _pair(dilation)
     cout, cin_g, kh, kw = weight.shape
     b = x.shape[0]
-    cols, ho, wo = _columns(x, offset, mask, kh, kw, stride, padding, dilation, deformable_groups)
+    cols, ho, wo = _columns(x, offset, mask, kh, kw, stride, padding, dilation, deformable_groups, fp32_positions)
     cols = cols.reshape(b, groups, cin_g * kh * kw, ho * wo)
     wmat = weight.reshape(groups, cout // groups, cin_g * kh * kw)
     out = torch.einsum('gok,bgkp->bgop', wmat, cols).reshape(b, cout, ho, wo)
@@ -90,14 +108,14 @@ def modulated_deform_conv_oracle(x, offset, mask, weight, bias=None, stride=1, p
 
 
 def modulated_deform_conv_backward_oracle(x, offset, mask, weight, bias, grad_output, stride=1, padding=0,
-                                          dilation=1, groups=1, deformable_groups=1, dtype=None):
+                                          dilation=1, groups=1, deformable_groups=1, dtype=None, fp32_positions=False):
     """(grad_input, grad_offset, grad_mask, grad_weight, grad_bias) as returned by
-    ModulatedDeformConvFunction.backward (deform_conv.py:155-174)."""
+    ModulatedDeformConvFunction.backward (deform_conv.py:155-174).  fp32_positions: see sampling_positions."""
     dtype = dtype or x.dtype
     leaves = [t.detach().to(dtype).clone().requires_grad_(True) for t in (x, offset, mask, weight)]
     bl = None if bias is None else bias.detach().to(dtype).clone().requires_grad_(True)
     out = modulated_deform_conv_oracle(leaves[0], leaves[1], leaves[2], leaves[3], bl, stride, padding,
-                                       dilation, groups, deformable_groups, dtype)
+                                       dilation, groups, deformable_groups, dtype, fp32_positions)
     ins = leaves + ([bl] if bl is not None else [])
     grads = torch.autograd.grad(out, ins, grad_output.to(dtype), allow_unused=True)
     grads = [g if g is not None else torch.zeros_like(t) for g, t in zip(grads, ins)]

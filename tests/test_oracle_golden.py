@@ -132,3 +132,97 @@ def test_dcnv1_oracle(golden):
     gi, goff, _, gw, _ = oracle.modulated_deform_conv_backward_oracle(x, off, ones, w, None, g('go'), 1, 1, 1, groups, dg)
     for got, key in ((gi, 'gx'), (goff, 'goffset'), (gw, 'gweight')):
         assert (got - g(key)).abs().max().item() <= 2e-5 * max(1.0, g(key).abs().max().item()), key
+
+
+def _flip_problem(seed=0):
+    """A DCN problem (offsets ~ N(0, 2^2), dg 2, stride / dilation 1 and 2) in which a few offsets are -2^-25: at a base
+    position n >= 1, n - 2^-25 rounds to n in fp32, so those sampling points change cell between the exact and the
+    fp32 position."""
+    g = torch.Generator().manual_seed(seed)
+    b, c, h, w, dg = 2, 8, 9, 11, 2
+    x = torch.randn(b, c, h, w, generator=g)
+    off = torch.randn(b, 2 * dg * 9, h, w, generator=g) * 2
+    mask = torch.rand(b, dg * 9, h, w, generator=g)
+    wgt = torch.randn(6, c, 3, 3, generator=g)
+    bias = torch.randn(6, generator=g)
+    go = torch.randn(b, 6, h, w, generator=g)
+    off.view(-1)[torch.randperm(off.numel(), generator=g)[:40]] = -2.0 ** -25
+    return x, off, mask, wgt, bias, go, dg
+
+
+def test_dcn_oracle_fp32_positions_are_the_fp32_sums():
+    from oracle.dcn import sampling_positions
+    x, off, mask, wgt, bias, go, dg = _flip_problem()
+    for stride, pad, dil in ((1, 1, 1), (2, 2, 2)):
+        ho = (x.shape[2] + 2 * pad - (2 * dil + 1)) // stride + 1
+        wo = (x.shape[3] + 2 * pad - (2 * dil + 1)) // stride + 1
+        o = off[:, :, :ho, :wo].contiguous()
+        b = o.shape[0]
+        him, wim = sampling_positions(o.double(), 3, 3, (stride, stride), (pad, pad), (dil, dil), dg, torch.float64,
+                                      fp32_positions=True)
+        assert him.dtype == torch.float64 and him.shape == (b, dg, 9, ho, wo)
+        ov = o.view(b, dg, 9, 2, ho, wo)
+        ys = torch.arange(ho).view(ho, 1) * stride - pad
+        xs = torch.arange(wo).view(1, wo) * stride - pad
+        for k in range(9):
+            by = (ys + (k // 3) * dil).float()
+            bx = (xs + (k % 3) * dil).float()
+            assert torch.equal(him[:, :, k], (by + ov[:, :, k, 0]).double())       # torch's float32 sum, bit for bit
+            assert torch.equal(wim[:, :, k], (bx + ov[:, :, k, 1]).double())
+        # exact positions: the fp64 sum; the two differ by at most one fp32 rounding
+        ehim, _ = sampling_positions(o.double(), 3, 3, (stride, stride), (pad, pad), (dil, dil), dg, torch.float64)
+        assert (ehim - him).abs().max() <= 2.0 ** -24 * ehim.abs().max()
+    # straight-through: the derivative with respect to the offset is 1
+    o = off.double().requires_grad_(True)
+    him, wim = sampling_positions(o, 3, 3, (1, 1), (1, 1), (1, 1), dg, torch.float64, fp32_positions=True)
+    (him.sum() + 2 * wim.sum()).backward()
+    ov = o.grad.view(o.shape[0], dg, 9, 2, *o.shape[2:])
+    assert bool((ov[:, :, :, 0] == 1).all()) and bool((ov[:, :, :, 1] == 2).all())
+
+
+def test_dcn_oracle_fp32_positions_equal_exact_where_no_point_changes_cell():
+    """Both position definitions give the same forward and gradients, except grad_offset at the points whose cell the
+    fp32 rounding changes (the bilinear sample is continuous across a cell edge, its derivative is not)."""
+    from oracle.dcn import sampling_positions
+    x, off, mask, wgt, bias, go, dg = _flip_problem()
+    f64 = torch.float64
+    h, w = x.shape[2:]
+    hx, wx = sampling_positions(off.double(), 3, 3, (1, 1), (1, 1), (1, 1), dg, f64)
+    h32, w32 = sampling_positions(off.double(), 3, 3, (1, 1), (1, 1), (1, 1), dg, f64, fp32_positions=True)
+
+    def cell(y, x_):    # the cell a point reads, or -9 when it reads nothing
+        inside = (y > -1) & (x_ > -1) & (y < h) & (x_ < w)
+        return torch.where(inside, torch.floor(y), -9.0), torch.where(inside, torch.floor(x_), -9.0)
+    cy, cx = cell(hx, wx)
+    cy32, cx32 = cell(h32, w32)
+    flip = (cy != cy32) | (cx != cx32)                                  # [B, dg, 9, H, W]
+    assert 5 <= int(flip.sum()) <= 40
+    y = oracle.modulated_deform_conv_oracle(x, off, mask, wgt, bias, 1, 1, 1, 1, dg, dtype=f64)
+    y32 = oracle.modulated_deform_conv_oracle(x, off, mask, wgt, bias, 1, 1, 1, 1, dg, dtype=f64, fp32_positions=True)
+    assert (y - y32).abs().max() <= 1e-6 * y.abs().max()
+    ex = oracle.modulated_deform_conv_backward_oracle(x, off, mask, wgt, bias, go, 1, 1, 1, 1, dg, dtype=f64)
+    fp = oracle.modulated_deform_conv_backward_oracle(x, off, mask, wgt, bias, go, 1, 1, 1, 1, dg, dtype=f64,
+                                                      fp32_positions=True)
+    for a, r, name in zip(fp, ex, ('input', 'offset', 'mask', 'weight', 'bias')):
+        if name == 'offset':
+            keep = ~flip.unsqueeze(3).expand(-1, -1, -1, 2, -1, -1).reshape(a.shape)
+            assert (a - r)[keep].abs().max() <= 1e-6 * r.abs().max(), name
+            assert (a - r)[~keep].abs().max() >= 1e-2 * r.abs().max(), name      # and the flips do show
+        else:
+            assert (a - r).abs().max() <= 1e-6 * r.abs().max(), name
+
+
+@pytest.mark.parametrize('case', ['small', 'big_offsets'])
+def test_dcn_oracle_fp32_positions_golden(golden, case):
+    """The reference's own gradients, which come from fp32 positions, are matched with the option on too."""
+    g = golden('dynagg')
+    dg = int(g(f'{case}.dg'))
+    x, off, mask, w, b = (g(f'{case}.{k}') for k in ('x', 'offset', 'mask', 'weight', 'bias'))
+    y = oracle.modulated_deform_conv_oracle(x, off, mask, w, b, 1, 1, 1, 1, dg, dtype=torch.float64, fp32_positions=True)
+    ref = g(f'{case}.y')
+    assert (y - ref).abs().max().item() <= 1e-5 * ref.abs().max().item()
+    grads = oracle.modulated_deform_conv_backward_oracle(x, off, mask, w, b, g(f'{case}.go'), 1, 1, 1, 1, dg,
+                                                         dtype=torch.float64, fp32_positions=True)
+    for got, key in zip(grads, ('gx', 'goffset', 'gmask', 'gweight', 'gbias')):
+        r = g(f'{case}.{key}')
+        assert (got - r).abs().max().item() <= 2e-5 * max(1.0, r.abs().max().item()), key
