@@ -108,12 +108,15 @@ MREFSR_API int mrefsr_pre_offsets(const int64_t* max_idx, int n, int h, int w, f
  * replaced by `workspace`.
  * mask == NULL means an all-ones mask: with bias == NULL that is DCNv1 (deform_conv_forward,
  * deform_conv_ext.cpp:52-66; same sampling rule, deform_conv_cuda_kernel.cu:84-112, 190-243).
- * mode: MREFSR_DCN_AUTO / MREFSR_DCN_FP32 (CUDA-core, exact fp32) / MREFSR_DCN_TF32 (tcgen05).
+ * mode: MREFSR_DCN_AUTO / MREFSR_DCN_FP32 (CUDA-core, exact fp32) / MREFSR_DCN_TF32 (tcgen05) /
+ *       MREFSR_DCN_TF32X3 (tcgen05 with 3-pass split-tf32 operands, hi.hi + hi.lo + lo.hi: fp32-grade results, same
+ *       shapes as MREFSR_DCN_TF32; in the backward it applies to the two GEMMs that MREFSR_DCN_TF32 runs on tcgen05).
  * ------------------------------------------------------------------------------------------ */
 enum {
     MREFSR_DCN_AUTO = 0,
     MREFSR_DCN_FP32 = 1,
     MREFSR_DCN_TF32 = 2,
+    MREFSR_DCN_TF32X3 = 3,
 };
 MREFSR_API size_t mrefsr_dcn_workspace_bytes(int B, int C, int H, int W, int Co, int kh, int kw, int stride_h, int stride_w,
                                   int pad_h, int pad_w, int dil_h, int dil_w, int group, int deformable_group,
@@ -177,6 +180,9 @@ enum {
     MREFSR_DCN_IN_NHWC = 1,
     MREFSR_DCN_OUT_NHWC = 2,
     MREFSR_DCN_W_PACKED = 4, /* `weight` is the output of mrefsr_dcn_pack_weights (inference: packed once per weight update) */
+    MREFSR_DCN_X3 = 8,       /* 3-pass split-tf32 operands (as mode MREFSR_DCN_TF32X3); with MREFSR_DCN_W_PACKED the
+                                weight must come from mrefsr_dcn_pack_weights_x3; workspace: mrefsr_dcn_workspace_bytes
+                                with mode MREFSR_DCN_TF32X3 */
 };
 /* The plain GEMM of the DCN backward on tcgen05 (csrc/gemm_tc.cu; TF32 operands, fp32 accumulate), exported for tests:
  *   D[m][n] = sum_k A[m][k] * B[n][k],   A [M x K] and B [N x K] row-major (k contiguous), D row-major with pitch ldd.
@@ -189,10 +195,20 @@ enum {
 MREFSR_API int mrefsr_gemm_tf32_nt(const float* A, int lda, long long a_batch_stride, const float* B, int ldb,
                                    long long b_batch_stride, float* D, int ldd, long long d_stride, int M, int N, int K,
                                    int batch, int reduce, int splits, void* stream);
+/* The same GEMM with 3-pass split-tf32 operands (the backward of mode MREFSR_DCN_TF32X3): each operand comes as a tf32 hi
+ * plane and a tf32 lo plane (x = hi + lo, both with the same pitch and batch stride), and
+ *   D = A_lo . B_hi^T + A_hi . B_lo^T + A_hi . B_hi^T   accumulated in fp32 (fp32-grade products; A_lo . B_lo^T is dropped). */
+MREFSR_API int mrefsr_gemm_tf32x3_nt(const float* A_hi, const float* A_lo, int lda, long long a_batch_stride,
+                                     const float* B_hi, const float* B_lo, int ldb, long long b_batch_stride, float* D,
+                                     int ldd, long long d_stride, int M, int N, int K, int batch, int reduce, int splits,
+                                     void* stream);
 /* W[Co][C][kh*kw] (the reference's parameter layout, deform_conv.py:305-309) -> the tcgen05 kernels' B operand
  * [Co][tap][C], rounded to tf32 (round to nearest, so the tensor core's truncation is exact).  The forward entry
  * points do this on every call unless MREFSR_DCN_W_PACKED is set; a module whose weights are frozen packs once. */
 MREFSR_API int mrefsr_dcn_pack_weights(const float* weight, float* packed, int Co, int C, int K, void* stream);
+/* The B operand of the 3-pass kernels (MREFSR_DCN_X3): [Co][tap][C/16][hi c0..7 | hi c8..15 | lo c0..7 | lo c8..15],
+ * 2*K*C floats per output channel, hi = tf32(w), lo = tf32(w - hi).  C % 16 == 0. */
+MREFSR_API int mrefsr_dcn_pack_weights_x3(const float* weight, float* packed, int Co, int C, int K, void* stream);
 MREFSR_API int mrefsr_dynagg_dcn_forward_ex(const float* input, const float* weight, const float* bias,
                                  const float* conv_out, const int64_t* max_idx, int flow_scale, float* output, int B,
                                  int C, int H, int W, int Co, int deformable_group, int with_bias, int layout_flags,

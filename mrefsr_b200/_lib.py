@@ -31,7 +31,10 @@ SIGNATURES = {
     'mrefsr_modulated_deform_conv_backward': (c_int, [_P] * 10 + [_I] * 17 + [_P, c_size_t, _P]),
     'mrefsr_gemm_tf32_nt': (c_int, [_P, _I, ctypes.c_longlong, _P, _I, ctypes.c_longlong, _P, _I, ctypes.c_longlong,
                                     _I, _I, _I, _I, _I, _I, _P]),
+    'mrefsr_gemm_tf32x3_nt': (c_int, [_P, _P, _I, ctypes.c_longlong, _P, _P, _I, ctypes.c_longlong, _P, _I,
+                                      ctypes.c_longlong, _I, _I, _I, _I, _I, _I, _P]),
     'mrefsr_dcn_pack_weights': (c_int, [_P, _P, _I, _I, _I, _P]),
+    'mrefsr_dcn_pack_weights_x3': (c_int, [_P, _P, _I, _I, _I, _P]),
     'mrefsr_dynagg_dcn_forward': (c_int, [_P] * 5 + [_I] + [_P] + [_I] * 7 + [_P, c_size_t, _P]),
     'mrefsr_dynagg_dcn_forward_multi': (c_int, [_P] * 5 + [_I] + [_P] + [_I] * 12 + [ctypes.c_float, _P, c_size_t, _P]),
     'mrefsr_dynagg_dcn_forward_slabs': (c_int, [_P] * 5 + [_I] + [_P] + [_I] * 13 + [ctypes.c_float, _P, c_size_t, _P]),

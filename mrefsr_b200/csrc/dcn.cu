@@ -329,10 +329,12 @@ dcn_bwd_coord_nhwc_kernel(const float* __restrict__ xt, const float* __restrict_
 // points, so when a backward wants both (grad_offset / grad_mask and grad_weight: every training step of MRefSR) one kernel
 // gathers them once.  Thread = (bl, deform group, position), taps as a loop; columns are written as planes
 // colT[bl][tap*C + c][p], rounded to tf32 (the grad_weight GEMM's B operand), exactly where dcn_im2col_planes_kernel puts them.
+// X3: colT gets tf32(col) and colT_lo the remainder tf32(col - tf32(col)) at the same index (3-pass GEMM operand planes).
+template <bool X3>
 __global__ void __launch_bounds__(256, 3)
 dcn_bwd_coord_cols_kernel(const float* __restrict__ xt, const float* __restrict__ offset, const float* __restrict__ mask,
                           const float* __restrict__ gcol, float* __restrict__ goff, float* __restrict__ gmask,
-                          float* __restrict__ colT, const DcnShape s, int b0, int nb) {
+                          float* __restrict__ colT, const DcnShape s, int b0, int nb, float* __restrict__ colT_lo) {
     const int K = s.kh * s.kw, P = s.Ho * s.Wo, cdg = s.C / s.DG;
     const size_t total = (size_t)nb * s.DG * P;
     for (size_t idx = (size_t)blockIdx.x * blockDim.x + threadIdx.x; idx < total; idx += (size_t)gridDim.x * blockDim.x) {
@@ -350,7 +352,8 @@ dcn_bwd_coord_cols_kernel(const float* __restrict__ xt, const float* __restrict_
             const float x = (float)(ox * s.sw - s.pw + tj * s.dw) + __ldcs(offset + ob + P);
             const float m = mask ? __ldcs(mask + mb) : 1.f;
             float dy = 0.f, dx = 0.f, dm = 0.f;
-            float* ct = colT + ((size_t)bl * K * s.C + (size_t)tap * s.C + dgi * cdg) * P + p;
+            const size_t ct_off = ((size_t)bl * K * s.C + (size_t)tap * s.C + dgi * cdg) * P + p;
+            float* ct = colT + ct_off;
             if (y > -1.f && x > -1.f && y < (float)s.H && x < (float)s.W) {
                 const float fy0 = floorf(y), fx0 = floorf(x);
                 const int y0 = (int)fy0, x0 = (int)fx0;
@@ -375,11 +378,16 @@ dcn_bwd_coord_cols_kernel(const float* __restrict__ xt, const float* __restrict_
                         dy += g * m * (hx * (cq - a) + lx * (d - bq));
                         dx += g * m * (hy * (bq - a) + ly * (d - cq));
                         // the column exactly as dcn_im2col_planes_kernel computes it (mask and validity folded into the weights)
-                        __stcs(ct + (size_t)(c0 + e) * P, to_tf32(w0 * v0.v[e] + w1 * v1.v[e] + w2 * v2.v[e] + w3 * v3.v[e]));
+                        const float col = w0 * v0.v[e] + w1 * v1.v[e] + w2 * v2.v[e] + w3 * v3.v[e], hi = to_tf32(col);
+                        __stcs(ct + (size_t)(c0 + e) * P, hi);
+                        if (X3) __stcs(colT_lo + ct_off + (size_t)(c0 + e) * P, to_tf32(col - hi));
                     }
                 }
             } else {
-                for (int c = 0; c < cdg; ++c) __stcs(ct + (size_t)c * P, 0.f);
+                for (int c = 0; c < cdg; ++c) {
+                    __stcs(ct + (size_t)c * P, 0.f);
+                    if (X3) __stcs(colT_lo + ct_off + (size_t)c * P, 0.f);
+                }
             }
             __stcs(goff + ob, dy);
             __stcs(goff + ob + P, dx);
@@ -390,10 +398,11 @@ dcn_bwd_coord_cols_kernel(const float* __restrict__ xt, const float* __restrict_
 
 // written as planes colT[bl][tap*C + c][p] (k = position contiguous: the B operand of the
 // tcgen05 grad_weight GEMM).  Lanes = consecutive positions, so each of the 8 scalar stores of a thread is a coalesced
-// 128-byte warp store into its channel plane.
+// 128-byte warp store into its channel plane.  X3: colT_lo receives the tf32 remainders (as in dcn_bwd_coord_cols_kernel).
+template <bool X3>
 __global__ void __launch_bounds__(256)
 dcn_im2col_planes_kernel(const float* __restrict__ xt, const float* __restrict__ offset, const float* __restrict__ mask,
-                         float* __restrict__ colT, const DcnShape s, int b0, int nb) {
+                         float* __restrict__ colT, const DcnShape s, int b0, int nb, float* __restrict__ colT_lo) {
     // thread = (bl, 8-channel chunk, position), taps as a loop (their corners meet in L1, as in the coordinate kernel)
     const int K = s.kh * s.kw, P = s.Ho * s.Wo, cdg = s.C / s.DG, C8 = s.C >> 3;
     const size_t total = (size_t)nb * C8 * P;
@@ -425,25 +434,37 @@ dcn_im2col_planes_kernel(const float* __restrict__ xt, const float* __restrict__
 #pragma unroll
                 for (int e = 0; e < 8; ++e) o[e] = w0 * v0.v[e] + w1 * v1.v[e] + w2 * v2.v[e] + w3 * v3.v[e];
             }
-            float* dst = colT + ((size_t)bl * K * s.C + (size_t)tap * s.C + c0) * P + p;
+            const size_t d_off = ((size_t)bl * K * s.C + (size_t)tap * s.C + c0) * P + p;
 #pragma unroll
-            for (int e = 0; e < 8; ++e) __stcs(dst + (size_t)e * P, to_tf32(o[e]));     // GEMM operand: the tensor core's read truncates
+            for (int e = 0; e < 8; ++e) {
+                const float hi = to_tf32(o[e]);              // GEMM operand: the tensor core's read truncates
+                __stcs(colT + d_off + (size_t)e * P, hi);
+                if (X3) __stcs(colT_lo + d_off + (size_t)e * P, to_tf32(o[e] - hi));
+            }
         }
     }
 }
 
-__global__ void dcn_weight_transpose_kernel(const float* __restrict__ w, float* __restrict__ wT, int Co, int MK) {
+// (wT_lo / dst_lo non-NULL: also the tf32 remainder, the lo plane of a 3-pass GEMM operand)
+__global__ void dcn_weight_transpose_kernel(const float* __restrict__ w, float* __restrict__ wT, int Co, int MK,
+                                            float* __restrict__ wT_lo) {
     const int total = Co * MK;
     for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < total; i += gridDim.x * blockDim.x) {
         const int oc = i % Co, m = i / Co;
-        wT[i] = to_tf32(__ldg(w + (size_t)oc * MK + m));
+        const float v = __ldg(w + (size_t)oc * MK + m), hi = to_tf32(v);
+        wT[i] = hi;
+        if (wT_lo) wT_lo[i] = to_tf32(v - hi);
     }
 }
 
 // tf32-rounded copy (GEMM operand whose natural layout is already the one the GEMM wants)
-__global__ void dcn_round_tf32_kernel(const float* __restrict__ src, float* __restrict__ dst, size_t n) {
-    for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (size_t)gridDim.x * blockDim.x)
-        dst[i] = to_tf32(__ldg(src + i));
+__global__ void dcn_round_tf32_kernel(const float* __restrict__ src, float* __restrict__ dst, size_t n,
+                                      float* __restrict__ dst_lo) {
+    for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (size_t)gridDim.x * blockDim.x) {
+        const float v = __ldg(src + i), hi = to_tf32(v);
+        dst[i] = hi;
+        if (dst_lo) dst_lo[i] = to_tf32(v - hi);
+    }
 }
 
 // gwT[i] += sum over the splits of part[s][i], in split order (deterministic)
@@ -692,9 +713,11 @@ int dcn_make_shape(DcnShape* s, int B, int C, int H, int W, int Co, int kh, int 
 
 constexpr int BWD_MAX_SPLITS = 32;     // split-K pieces of the grad_weight GEMM (partial sums in the workspace)
 
-static int bwd_chunk(const DcnShape& s) {
+static int bwd_chunk(const DcnShape& s, bool x3) {
     const size_t per = (size_t)s.C * s.kh * s.kw * s.Ho * s.Wo * 4;
-    size_t nb = ((size_t)1024 << 20) / per;     // two scratch tensors of <= 1 GiB (columns, their gradient): fewer, larger launches
+    // two scratch tensors of <= 1 GiB (columns, their gradient): fewer, larger launches.  The 3-pass mode adds the
+    // columns' lo plane and keeps the three within the same 2 GiB.
+    size_t nb = (x3 ? ((size_t)2048 << 20) / 3 : ((size_t)1024 << 20)) / per;
     if (nb < 1) nb = 1;
     if (nb > (size_t)s.B) nb = s.B;
     return (int)nb;
@@ -736,12 +759,15 @@ size_t mrefsr_dcn_workspace_bytes(int B, int C, int H, int W, int Co, int kh, in
     if (dcn_make_shape(&s, B, C, H, W, Co, kh, kw, stride_h, stride_w, pad_h, pad_w, dil_h, dil_w, group,
                        deformable_group))
         return 0;
-    if (backward)   // gcol + col chunks, NHWC copies of the input and of grad_output, W^T, tap-major grad_weight scratch
-                    // and the split-K partial sums of the grad_weight GEMM
-        return 2 * align_up((size_t)bwd_chunk(s) * C * kh * kw * s.Ho * s.Wo * 4, 1024) +
-               align_up((size_t)B * C * H * W * 4, 1024) + 2 * align_up((size_t)B * Co * s.Ho * s.Wo * 4, 1024) +
-               2 * align_up((size_t)Co * C * kh * kw * 4, 1024) +
-               align_up((size_t)BWD_MAX_SPLITS * Co * C * kh * kw * 4, 1024) + 1024;
+    if (backward) { // gcol + col chunks, NHWC copies of the input and of grad_output, W^T, tap-major grad_weight scratch
+                    // and the split-K partial sums of the grad_weight GEMM; the 3-pass mode adds the lo planes of the
+                    // GEMM operands (col, both copies of grad_output, W^T)
+        const bool x3 = mode == MREFSR_DCN_TF32X3;
+        const size_t buf = align_up((size_t)bwd_chunk(s, x3) * C * kh * kw * s.Ho * s.Wo * 4, 1024);
+        const size_t got = align_up((size_t)B * Co * s.Ho * s.Wo * 4, 1024), gwt = align_up((size_t)Co * C * kh * kw * 4, 1024);
+        return 2 * buf + align_up((size_t)B * C * H * W * 4, 1024) + 2 * got + 2 * gwt +
+               align_up((size_t)BWD_MAX_SPLITS * Co * C * kh * kw * 4, 1024) + (x3 ? buf + 2 * got + gwt : 0) + 1024;
+    }
     return dcn_tc_workspace_bytes(s, mode) + 1024;
 }
 
@@ -761,11 +787,12 @@ int mrefsr_modulated_deform_conv_forward(const float* input, const float* weight
     int m = mode;
     if (m == MREFSR_DCN_AUTO) m = dcn_tc_eligible(s) ? MREFSR_DCN_TF32 : MREFSR_DCN_FP32;
     if (m == MREFSR_DCN_FP32) return dcn_forward_fp32(input, weight, bp, offset, mask, output, s, st);
-    MREFSR_CHECK(m == MREFSR_DCN_TF32, ERR_BAD_ARG, "dcn forward: unknown mode %d", mode);
+    MREFSR_CHECK(m == MREFSR_DCN_TF32 || m == MREFSR_DCN_TF32X3, ERR_BAD_ARG, "dcn forward: unknown mode %d", mode);
     MREFSR_CHECK(dcn_tc_eligible(s), ERR_UNSUPPORTED,
                  "dcn forward: tcgen05 path needs group 1, C %% 32 == 0, Co %% 32 == 0, Co <= 256, "
                  "(C/deformable_group) %% 4 == 0");
-    return dcn_forward_tc(input, weight, bp, offset, mask, output, s, workspace, workspace_bytes, st);
+    return dcn_forward_tc(input, weight, bp, offset, mask, output, s, workspace, workspace_bytes, st,
+                          m == MREFSR_DCN_TF32X3);
 }
 
 int mrefsr_modulated_deform_conv_backward(const float* input, const float* weight, const float* offset,
@@ -780,6 +807,8 @@ int mrefsr_modulated_deform_conv_backward(const float* input, const float* weigh
     // (gemm_tc.cu, TF32 operands, fp32 accumulate) whenever the operand pitches allow TMA (group 1, Co % 4 == 0 for
     // the columns GEMM, output positions % 4 == 0 for the grad_weight GEMM)
     const bool tc_gemm = mode != MREFSR_DCN_FP32;
+    // MREFSR_DCN_TF32X3: those two GEMMs take hi / lo operand planes and run the 3-pass kernel (fp32-grade products)
+    const bool x3 = mode == MREFSR_DCN_TF32X3;
     MREFSR_CHECK(grad_offset || !grad_mask, ERR_BAD_ARG, "dcn backward: grad_mask requires grad_offset");
     MREFSR_CHECK(!with_bias || grad_bias, ERR_BAD_ARG, "dcn backward: with_bias set but grad_bias is NULL");
     DcnShape s;
@@ -788,7 +817,7 @@ int mrefsr_modulated_deform_conv_backward(const float* input, const float* weigh
     if (rc) return rc;
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     const int K = kh * kw, P = s.Ho * s.Wo, cpg = C / group, opg = Co / group, MK = cpg * K;
-    const int nbmax = bwd_chunk(s);
+    const int nbmax = bwd_chunk(s, x3);
     const size_t buf = align_up((size_t)nbmax * C * K * P * 4, 1024);
     const size_t xt_bytes = align_up((size_t)B * C * H * W * 4, 1024), gwt_bytes = align_up((size_t)Co * C * K * 4, 1024);
     const size_t got_bytes = align_up((size_t)B * Co * P * 4, 1024);
@@ -800,8 +829,9 @@ int mrefsr_modulated_deform_conv_backward(const float* input, const float* weigh
     const bool tc_gw = tc_gemm && grad_weight && group == 1 && C % 8 == 0 && (C / deformable_group) % 8 == 0 && P % 4 == 0 &&
                        small_enough;
     const size_t need = 2 * buf + xt_bytes + 2 * got_bytes + 2 * gwt_bytes + part_bytes;
-    MREFSR_CHECK(workspace && workspace_bytes >= need, ERR_WORKSPACE, "dcn backward: workspace too small (%zu < %zu)",
-                 workspace_bytes, need);
+    const size_t need_all = need + (x3 ? buf + 2 * got_bytes + gwt_bytes : 0);
+    MREFSR_CHECK(workspace && workspace_bytes >= need_all, ERR_WORKSPACE, "dcn backward: workspace too small (%zu < %zu)",
+                 workspace_bytes, need_all);
     MREFSR_CHECK((reinterpret_cast<uintptr_t>(workspace) & 1023) == 0, ERR_WORKSPACE, "dcn backward: workspace must be 1024-byte aligned");
     uint8_t* wsp = static_cast<uint8_t*>(workspace);
     float* gcol = reinterpret_cast<float*>(wsp);
@@ -812,6 +842,12 @@ int mrefsr_modulated_deform_conv_backward(const float* input, const float* weigh
     float* wT = reinterpret_cast<float*>(wsp + 2 * buf + xt_bytes + got_bytes + gwt_bytes);
     float* part = reinterpret_cast<float*>(wsp + 2 * buf + xt_bytes + got_bytes + 2 * gwt_bytes);
     float* goutR = reinterpret_cast<float*>(wsp + 2 * buf + xt_bytes + got_bytes + 2 * gwt_bytes + part_bytes);
+    // lo planes of the 3-pass GEMM operands, after the buffers above (counted by mrefsr_dcn_workspace_bytes for mode 3)
+    uint8_t* lo_base = wsp + need;
+    float* col_lo = x3 ? reinterpret_cast<float*>(lo_base) : nullptr;
+    float* goutT_lo = x3 ? reinterpret_cast<float*>(lo_base + buf) : nullptr;
+    float* goutR_lo = x3 ? reinterpret_cast<float*>(lo_base + buf + got_bytes) : nullptr;
+    float* wT_lo = x3 ? reinterpret_cast<float*>(lo_base + buf + 2 * got_bytes) : nullptr;
     // grad_offset / grad_mask from the NHWC copy (four 256-bit corner loads per 8-channel chunk instead of 32 scalar loads)
     const bool nhwc_coord = tc_gemm && grad_offset && C % 8 == 0 && (C / deformable_group) % 8 == 0 && small_enough;
     if (tc_gw || nhwc_coord) {
@@ -820,14 +856,14 @@ int mrefsr_modulated_deform_conv_backward(const float* input, const float* weigh
     }
     if (tc_gw) {
         MREFSR_CUDA(cudaMemsetAsync(gwT, 0, (size_t)Co * C * K * 4, st));
-        dcn_round_tf32_kernel<<<grid_for((size_t)B * Co * P), 256, 0, st>>>(grad_output, goutR, (size_t)B * Co * P);
+        dcn_round_tf32_kernel<<<grid_for((size_t)B * Co * P), 256, 0, st>>>(grad_output, goutR, (size_t)B * Co * P, goutR_lo);
         MREFSR_LAUNCH_CHECK();
         count_launches(1);
     }
     if (tc_gcol) {
-        rc = dcn_nchw_to_nhwc(grad_output, goutT, B, Co, P, st, true);
+        rc = dcn_nchw_to_nhwc(grad_output, goutT, B, Co, P, st, true, goutT_lo);
         if (rc) return rc;
-        dcn_weight_transpose_kernel<<<cdiv(Co * MK, 256), 256, 0, st>>>(weight, wT, Co, MK);
+        dcn_weight_transpose_kernel<<<cdiv(Co * MK, 256), 256, 0, st>>>(weight, wT, Co, MK, wT_lo);
         MREFSR_LAUNCH_CHECK();
         count_launches(1);
     }
@@ -837,7 +873,7 @@ int mrefsr_modulated_deform_conv_backward(const float* input, const float* weigh
         if (tc_gcol) {
             // (deform_conv_cuda.cpp:623-626), all samples of the chunk in one launch
             rc = gemm_tf32_nt(wT, Co, 0, goutT + (size_t)b0 * P * Co, Co, (long long)P * Co, gcol, P, (long long)MK * P, MK, P,
-                              Co, nb, 0, 1, st);
+                              Co, nb, 0, 1, st, wT_lo, x3 ? goutT_lo + (size_t)b0 * P * Co : nullptr);
             if (rc) return rc;
         } else if (grad_input || grad_offset) {
             dcn_bwd_gcol_kernel<<<dim3(cdiv(P, DT), group * cdiv(MK, DT), nb), 256, 0, st>>>(weight, grad_output, gcol, s, b0);
@@ -847,8 +883,12 @@ int mrefsr_modulated_deform_conv_backward(const float* input, const float* weigh
         // coordinate gradients and recomputed columns from ONE gather when the backward wants both
         const bool merged = grad_offset && nhwc_coord && tc_gw;
         if (merged) {
-            dcn_bwd_coord_cols_kernel<<<grid_for((size_t)nb * deformable_group * P), 256, 0, st>>>(
-                xt, offset, mask, gcol, grad_offset, grad_mask, col, s, b0, nb);
+            if (x3)
+                dcn_bwd_coord_cols_kernel<true><<<grid_for((size_t)nb * deformable_group * P), 256, 0, st>>>(
+                    xt, offset, mask, gcol, grad_offset, grad_mask, col, s, b0, nb, col_lo);
+            else
+                dcn_bwd_coord_cols_kernel<false><<<grid_for((size_t)nb * deformable_group * P), 256, 0, st>>>(
+                    xt, offset, mask, gcol, grad_offset, grad_mask, col, s, b0, nb, nullptr);
             MREFSR_LAUNCH_CHECK();
             count_launches(1);
         } else if (grad_offset && nhwc_coord) {
@@ -871,7 +911,12 @@ int mrefsr_modulated_deform_conv_backward(const float* input, const float* weigh
             // recomputed columns (deform_conv_cuda.cpp:647-650) as planes colT[bl][tap*C + c][p], then the chunk's share
             // of grad_weight (:659-664) as one split-K GEMM whose partial sums are added up in a fixed order
             if (!merged) {
-                dcn_im2col_planes_kernel<<<grid_for((size_t)nb * (C / 8) * P), 256, 0, st>>>(xt, offset, mask, col, s, b0, nb);
+                if (x3)
+                    dcn_im2col_planes_kernel<true><<<grid_for((size_t)nb * (C / 8) * P), 256, 0, st>>>(xt, offset, mask, col, s,
+                                                                                                      b0, nb, col_lo);
+                else
+                    dcn_im2col_planes_kernel<false><<<grid_for((size_t)nb * (C / 8) * P), 256, 0, st>>>(xt, offset, mask, col, s,
+                                                                                                       b0, nb, nullptr);
                 MREFSR_LAUNCH_CHECK();
                 count_launches(1);
             }
@@ -882,7 +927,8 @@ int mrefsr_modulated_deform_conv_backward(const float* input, const float* weigh
             if (splits > all_kb) splits = (int)all_kb;
             if (splits < 1) splits = 1;
             rc = gemm_tf32_nt(goutR + (size_t)b0 * Co * P, P, (long long)Co * P, col, P, (long long)K * C * P, part, K * C,
-                              (long long)Co * K * C, Co, K * C, P, nb, 1, splits, st);
+                              (long long)Co * K * C, Co, K * C, P, nb, 1, splits, st,
+                              x3 ? goutR_lo + (size_t)b0 * Co * P : nullptr, col_lo);
             if (rc) return rc;
             dcn_split_sum_kernel<<<cdiv(Co * C * K, 256), 256, 0, st>>>(part, gwT, Co * C * K, splits);
             MREFSR_LAUNCH_CHECK();
@@ -920,9 +966,23 @@ int mrefsr_gemm_tf32_nt(const float* A, int lda, long long a_batch_stride, const
                         static_cast<cudaStream_t>(stream));
 }
 
+int mrefsr_gemm_tf32x3_nt(const float* A_hi, const float* A_lo, int lda, long long a_batch_stride, const float* B_hi,
+                          const float* B_lo, int ldb, long long b_batch_stride, float* D, int ldd, long long d_stride, int M,
+                          int N, int K, int batch, int reduce, int splits, void* stream) {
+    MREFSR_CHECK(A_hi && A_lo && B_hi && B_lo && D, ERR_BAD_ARG, "gemm (x3): null pointer argument");
+    MREFSR_CHECK(!reduce || splits >= 1, ERR_BAD_ARG, "gemm (x3): reduce mode needs splits >= 1");
+    return gemm_tf32_nt(A_hi, lda, a_batch_stride, B_hi, ldb, b_batch_stride, D, ldd, d_stride, M, N, K, batch, reduce,
+                        splits, static_cast<cudaStream_t>(stream), A_lo, B_lo);
+}
+
 int mrefsr_dcn_pack_weights(const float* weight, float* packed, int Co, int C, int K, void* stream) {
     MREFSR_CHECK(weight && packed && Co > 0 && C > 0 && K > 0, ERR_BAD_ARG, "pack_weights: bad arguments");
     return dcn_pack_weights(weight, packed, Co, C, K, static_cast<cudaStream_t>(stream));
+}
+
+int mrefsr_dcn_pack_weights_x3(const float* weight, float* packed, int Co, int C, int K, void* stream) {
+    MREFSR_CHECK(weight && packed && Co > 0 && C > 0 && K > 0, ERR_BAD_ARG, "pack_weights_x3: bad arguments");
+    return dcn_pack_weights(weight, packed, Co, C, K, static_cast<cudaStream_t>(stream), true);
 }
 
 int mrefsr_dynagg_dcn_forward(const float* input, const float* weight, const float* bias, const float* conv_out,
@@ -947,7 +1007,7 @@ int mrefsr_dynagg_dcn_forward_ex(const float* input, const float* weight, const 
                                  void* workspace, size_t workspace_bytes, void* stream) {
     MREFSR_CHECK(input && weight && conv_out && max_idx && output, ERR_BAD_ARG, "dynagg forward: null pointer argument");
     MREFSR_CHECK(!with_bias || bias, ERR_BAD_ARG, "dynagg forward: with_bias set but bias is NULL");
-    MREFSR_CHECK((layout_flags & ~(MREFSR_DCN_IN_NHWC | MREFSR_DCN_OUT_NHWC | MREFSR_DCN_W_PACKED)) == 0, ERR_BAD_ARG,
+    MREFSR_CHECK((layout_flags & ~(MREFSR_DCN_IN_NHWC | MREFSR_DCN_OUT_NHWC | MREFSR_DCN_W_PACKED | MREFSR_DCN_X3)) == 0, ERR_BAD_ARG,
                  "dynagg forward: unknown layout flags 0x%x", layout_flags);
     DcnShape s;
     int rc = dcn_make_shape(&s, B, C, H, W, Co, 3, 3, 1, 1, 1, 1, 1, 1, 1, deformable_group);
@@ -966,7 +1026,7 @@ int mrefsr_dynagg_dcn_forward_multi(const float* input, const float* weight, con
                                     void* workspace, size_t workspace_bytes, void* stream) {
     MREFSR_CHECK(input && weight && conv_out && max_idx && outputs, ERR_BAD_ARG, "dynagg forward: null pointer argument");
     MREFSR_CHECK(!with_bias || bias, ERR_BAD_ARG, "dynagg forward: with_bias set but bias is NULL");
-    MREFSR_CHECK((layout_flags & ~(MREFSR_DCN_IN_NHWC | MREFSR_DCN_OUT_NHWC | MREFSR_DCN_W_PACKED)) == 0, ERR_BAD_ARG,
+    MREFSR_CHECK((layout_flags & ~(MREFSR_DCN_IN_NHWC | MREFSR_DCN_OUT_NHWC | MREFSR_DCN_W_PACKED | MREFSR_DCN_X3)) == 0, ERR_BAD_ARG,
                  "dynagg forward: unknown layout flags 0x%x", layout_flags);
     MREFSR_CHECK(n_outputs >= 1 && n_outputs <= 8, ERR_BAD_ARG, "dynagg forward: 1..8 output buffers (got %d)", n_outputs);
     DcnShape s;
@@ -993,7 +1053,7 @@ int mrefsr_dynagg_dcn_forward_slabs(const float* input, const float* weight, con
                                     void* workspace, size_t workspace_bytes, void* stream) {
     MREFSR_CHECK(input && weight && conv_out && max_idx && outputs, ERR_BAD_ARG, "dynagg forward: null pointer argument");
     MREFSR_CHECK(!with_bias || bias, ERR_BAD_ARG, "dynagg forward: with_bias set but bias is NULL");
-    MREFSR_CHECK((layout_flags & ~(MREFSR_DCN_IN_NHWC | MREFSR_DCN_W_PACKED)) == 0, ERR_BAD_ARG,
+    MREFSR_CHECK((layout_flags & ~(MREFSR_DCN_IN_NHWC | MREFSR_DCN_W_PACKED | MREFSR_DCN_X3)) == 0, ERR_BAD_ARG,
                  "dynagg forward (slabs): unknown or unsupported layout flags 0x%x", layout_flags);
     MREFSR_CHECK(n_outputs >= 1 && n_outputs <= 8 && slab_rows >= 1, ERR_BAD_ARG,
                  "dynagg forward (slabs): 1..8 output buffers and slab_rows >= 1 (got %d, %d)", n_outputs, slab_rows);

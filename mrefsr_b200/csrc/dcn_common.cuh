@@ -33,15 +33,18 @@ int dcn_forward_fp32(const float* x, const float* w, const float* bias, const fl
                      const DcnShape& s, cudaStream_t st);
 
 // NCHW -> NHWC copy (dcn_tc.cu), also used by the backward's position-major im2col
-int dcn_nchw_to_nhwc(const float* x, float* xt, int B, int C, int HW, cudaStream_t st, bool round_tf32 = false);
+// (xt_lo: the 3-pass split, xt = tf32(x) and xt_lo = tf32(x - xt))
+int dcn_nchw_to_nhwc(const float* x, float* xt, int B, int C, int HW, cudaStream_t st, bool round_tf32 = false,
+                     float* xt_lo = nullptr);
 
-// tcgen05 TF32 GEMM D = A . B^T of the backward pass (gemm_tc.cu)
+// tcgen05 TF32 GEMM D = A . B^T of the backward pass (gemm_tc.cu); A_lo / B_lo non-NULL: the 3-pass variant
+// D = A_lo . B^T + A . B_lo^T + A . B^T (A, B then hold the hi planes; the lo planes share their pitches and strides)
 bool gemm_tc_operands_ok(const void* A, int lda, long long a_batch_stride, const void* B, int ldb, long long b_batch_stride);
 int gemm_tf32_nt(const float* A, int lda, long long a_batch_stride, const float* B, int ldb, long long b_batch_stride,
                  float* D, int ldd, long long d_stride, int M, int N, int K, int batch, int reduce, int splits,
-                 cudaStream_t st);
+                 cudaStream_t st, const float* A_lo = nullptr, const float* B_lo = nullptr);
 
-int dcn_pack_weights(const float* w, float* wt, int Co, int C, int K, cudaStream_t st);
+int dcn_pack_weights(const float* w, float* wt, int Co, int C, int K, cudaStream_t st, bool x3 = false);
 
 // several destination buffers for one forward (reference-sharded mode: local + peer copies of the gathered tensor)
 struct DcnOutputs {
@@ -59,6 +62,6 @@ int dcn_forward_tc_impl(const float* x, const float* w, const float* bias, const
                         const DcnOutputs* multi);
 int dcn_tc_tile_plan(int B, int Ho, int Wo, int* meta, int* coords, size_t max_rows);
 int dcn_forward_tc(const float* x, const float* w, const float* bias, const float* off, const float* mask, float* out,
-                   const DcnShape& s, void* workspace, size_t workspace_bytes, cudaStream_t st);
+                   const DcnShape& s, void* workspace, size_t workspace_bytes, cudaStream_t st, bool x3);
 
 }  // namespace mrefsr

@@ -49,6 +49,10 @@
 // staged each patch's input window in shared memory by TMA gave the same bits and was slower on every flow kind
 // (same profile); it was removed (DESIGN.md 2.2b).
 //
+// The 3-pass mode (MREFSR_DCN_TF32X3 / the MREFSR_DCN_X3 flag, X3 = true instantiations) keeps this geometry and halves
+// the channels per K step: each 128-byte row holds the tf32 hi AND lo parts of 16 channels, and the MMA warp issues
+// lo.hi + hi.lo + hi.hi, which gives fp32-grade results at the price of twice the K steps (DESIGN.md 2.2).
+//
 // Offsets / masks come either as materialised tensors (the reference operator API) or -- fused DynAgg mode --
 // straight from the raw conv_offset_mask output plus the matcher's arg-max map: offset = conv + s*flow shifted
 // by the tap, mask = sigmoid(conv) (basicsr/archs/ref_mrapa_restoration_arch.py:55-68 and
@@ -64,9 +68,10 @@ namespace mrefsr {
 // NCHW -> NHWC (fp32): tile = 32 pixels x up to 128 channels per CTA (256 threads).  Loads: lane = pixel (128-byte
 // coalesced, 16 independent loads per thread in flight); stores: one float4 (4 channels) per lane, 512 bytes
 // contiguous per warp.  grid (ceil(HW/32), ceil(C/128), B)
-template <bool ROUND>     // ROUND: values rounded to tf32 on the way (operands of the tcgen05 GEMMs, whose reads truncate)
+template <bool ROUND,      // ROUND: values rounded to tf32 on the way (operands of the tcgen05 GEMMs, whose reads truncate)
+          bool SPLIT = false>   // SPLIT (with ROUND): dst gets tf32(v), dst_lo tf32(v - tf32(v)) (3-pass GEMM operands)
 __global__ void __launch_bounds__(256)
-nchw_to_nhwc_kernel(const float* __restrict__ src, float* __restrict__ dst, int C, int HW) {
+nchw_to_nhwc_kernel(const float* __restrict__ src, float* __restrict__ dst, int C, int HW, float* __restrict__ dst_lo) {
     __shared__ float tile[128][33];
     const int b = blockIdx.z, p0 = blockIdx.x * 32, c0 = blockIdx.y * 128;
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -77,7 +82,7 @@ nchw_to_nhwc_kernel(const float* __restrict__ src, float* __restrict__ dst, int 
     for (int i = 0; i < 16; ++i) {
         const int cl = warp + 8 * i, c = c0 + cl;
         const float v = (c < C && p < HW) ? __ldcs(s + (size_t)c * HW + p) : 0.f;
-        tile[cl][lane] = ROUND ? to_tf32(v) : v;
+        tile[cl][lane] = (ROUND && !SPLIT) ? to_tf32(v) : v;
     }
     __syncthreads();
 #pragma unroll
@@ -86,7 +91,14 @@ nchw_to_nhwc_kernel(const float* __restrict__ src, float* __restrict__ dst, int 
         if (pp < HW && c < C) {   // C % 4 == 0 on this path (C % 32 == 0 is an eligibility condition)
             const float4 v = make_float4(tile[lane * 4][pl], tile[lane * 4 + 1][pl], tile[lane * 4 + 2][pl],
                                          tile[lane * 4 + 3][pl]);
-            *reinterpret_cast<float4*>(d + (size_t)pp * C + c) = v;
+            if (SPLIT) {
+                const float4 h = make_float4(to_tf32(v.x), to_tf32(v.y), to_tf32(v.z), to_tf32(v.w));
+                *reinterpret_cast<float4*>(d + (size_t)pp * C + c) = h;
+                *reinterpret_cast<float4*>(dst_lo + (size_t)b * C * HW + (size_t)pp * C + c) =
+                    make_float4(to_tf32(v.x - h.x), to_tf32(v.y - h.y), to_tf32(v.z - h.z), to_tf32(v.w - h.w));
+            } else {
+                *reinterpret_cast<float4*>(d + (size_t)pp * C + c) = v;
+            }
         }
     }
 }
@@ -97,6 +109,19 @@ __global__ void dcn_weight_repack_kernel(const float* __restrict__ w, float* __r
     for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < total; i += gridDim.x * blockDim.x) {
         const int c = i % C, tap = (i / C) % K, co = i / (C * K);
         wt[i] = to_tf32(__ldg(w + ((size_t)co * C + c) * K + tap));
+    }
+}
+
+// W[co][c][tap] -> Wt[co][tap][C/16][hi c0..7 | hi c8..15 | lo c0..7 | lo c8..15]: the B operand of the 3-pass kernels,
+// one 128-byte TMA row per 16-channel slab (hi = tf32(w), lo = tf32(w - hi); cvt.rna clears the low bits)
+__global__ void dcn_weight_repack_x3_kernel(const float* __restrict__ w, float* __restrict__ wt, int Co, int C, int K) {
+    const int total = Co * C * K;
+    for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < total; i += gridDim.x * blockDim.x) {
+        const int c = i % C, tap = (i / C) % K, co = i / (C * K);
+        const float v = __ldg(w + ((size_t)co * C + c) * K + tap), hi = to_tf32(v);
+        float* o = wt + ((size_t)co * K + tap) * 2 * C + (c / TBK_X3) * 2 * TBK_X3 + c % TBK_X3;
+        o[0] = hi;
+        o[TBK_X3] = to_tf32(v - hi);
     }
 }
 
@@ -160,6 +185,9 @@ __device__ __forceinline__ void dcn_epilogue_tile(const DcnTcParams& prm, const 
 // MMA issuer (one elected thread of the MMA warp): per tile wait for a free TMEM accumulator, per K step wait for the
 // A / B stage, issue 2 (M halves) x 4 (K = 8) tcgen05.mma.kind::tf32, release the stage with a commit; a last commit
 // hands the accumulator to the epilogue warps.
+// X3: the stage holds [hi 16 | lo 16] channels of A and B; per M half and 8-channel step kk in {0, 1}: lo.hi, hi.lo,
+// hi.hi into the same accumulator (6 MMAs per 16 channels).
+template <bool X3>
 __device__ __forceinline__ void dcn_mma_issuer(const DcnTcParams& prm, uint8_t* smem, uint64_t* full, uint64_t* empty,
                                                uint64_t* tfull, uint64_t* tempty, uint32_t tmem_base, int nkb_tile) {
     const int Co = prm.s.Co, S = prm.stages;
@@ -178,15 +206,33 @@ __device__ __forceinline__ void dcn_mma_issuer(const DcnTcParams& prm, uint8_t* 
             tc_fence_after();
             const uint32_t sa = smem_u32(smem + (size_t)stage * prm.stage_bytes);
             const uint32_t sb = sa + T_A_BYTES;
+            if (X3) {
 #pragma unroll
-            for (int kk = 0; kk < 4; ++kk) {
+                for (int kk = 0; kk < 2; ++kk) {
 #ifdef MREFSR_DCN_DEBUG
-                if (prm.dbg & 8) continue;           // ablation 8: no MMAs
+                    if (prm.dbg & 8) continue;
 #endif
-                const uint64_t db = umma_desc_sw128(sb + kk * 32, 0);
-                umma_tf32(tacc, umma_desc_sw128(sa + kk * 32, 0), db, idesc, accumulate);
-                umma_tf32(tacc + Co, umma_desc_sw128(sa + 128 * 128 + kk * 32, 0), db, idesc, accumulate);
-                accumulate = 1;
+                    const uint64_t bh = umma_desc_sw128(sb + kk * 32, 0), bl = umma_desc_sw128(sb + (kk + 2) * 32, 0);
+#pragma unroll
+                    for (int half = 0; half < 2; ++half) {
+                        const uint32_t ah = sa + half * (128 * 128) + kk * 32;
+                        umma_tf32(tacc + half * Co, umma_desc_sw128(ah + 64, 0), bh, idesc, accumulate);
+                        umma_tf32(tacc + half * Co, umma_desc_sw128(ah, 0), bl, idesc, 1);
+                        umma_tf32(tacc + half * Co, umma_desc_sw128(ah, 0), bh, idesc, 1);
+                    }
+                    accumulate = 1;
+                }
+            } else {
+#pragma unroll
+                for (int kk = 0; kk < 4; ++kk) {
+#ifdef MREFSR_DCN_DEBUG
+                    if (prm.dbg & 8) continue;           // ablation 8: no MMAs
+#endif
+                    const uint64_t db = umma_desc_sw128(sb + kk * 32, 0);
+                    umma_tf32(tacc, umma_desc_sw128(sa + kk * 32, 0), db, idesc, accumulate);
+                    umma_tf32(tacc + Co, umma_desc_sw128(sa + 128 * 128 + kk * 32, 0), db, idesc, accumulate);
+                    accumulate = 1;
+                }
             }
             umma_commit(&empty[stage]);
             if (++stage == S) {
@@ -227,7 +273,13 @@ struct DcnRaw {                                     // inputs of one table row (
 // for its stage to be consumed, the other gathers.  Same arithmetic, same bits; measured on B200 (profiles/r02x):
 // 3.72 -> 3.36 ms per step on coherent flows, and with the groups decoupled a third stage pays at 16+ channels per
 // deform group (mid scale 0.93 -> 0.84 ms).
-template <bool FUSED, int GS>       // GS = deform groups per 32-channel slab (prm.gs: 1, 2 or 4)
+//
+// X3 (3-pass split-tf32, fp32-grade): same stage geometry, but a K step covers a 16-channel slab whose 128-byte rows
+// are [hi c0..7 | hi c8..15 | lo c0..7 | lo c8..15]; a gather thread then owns two (row, 8-channel chunk) items per
+// K step instead of four, the MMA warp issues lo.hi + hi.lo + hi.hi, and the weights come packed the same way
+// (dcn_weight_repack_x3_kernel).  The stage bytes, stage count and TMEM use are those of the tf32 kernel.
+template <bool FUSED, int GS,       // GS = deform groups per slab (prm.gs: 1, 2 or 4; X3: 1 or 2)
+          bool X3 = false>
 __global__ void __launch_bounds__(S_THREADS, 1)
 dcn_tc_split_kernel(const __grid_constant__ CUtensorMap mapW, const float* __restrict__ xt,
                     const float* __restrict__ offset, const float* __restrict__ mask,
@@ -279,13 +331,19 @@ dcn_tc_split_kernel(const __grid_constant__ CUtensorMap mapW, const float* __res
 
     if (warp < S_GW) {
         // ------------------------------------------------------------------ gather warps, two groups on alternate K steps
+        constexpr int SLAB = X3 ? TBK_X3 : TBK;    // channels per K step
+        constexpr int ITEMS = X3 ? 2 : 4;          // (row, 8-channel chunk) items per thread and K step
+        constexpr int RSTEP = TBM / ITEMS;         // row distance between a thread's items
         const int grp = warp >> 3;                 // this group's K steps: kb = grp (mod 2)
         const int tg = threadIdx.x & 255;          // thread within the group
-        const int ch = tg & 3;                     // 8-channel chunk within the 32-channel slab
-        const int r0 = tg >> 2;                    // rows r0 + 64 i, i < 4
+        const int ch = tg & (SLAB / 8 - 1);        // 8-channel chunk within the slab
+        const int r0 = tg >> (X3 ? 1 : 2);         // rows r0 + RSTEP i, i < ITEMS
         const int gsub = (ch * 8) / prm.cdg;
         const uint32_t a_off0 = (uint32_t)r0 * 128u + (uint32_t)(((2 * ch) ^ (r0 & 7)) << 4);
         const uint32_t a_off1 = (uint32_t)r0 * 128u + (uint32_t)(((2 * ch + 1) ^ (r0 & 7)) << 4);
+        // X3: the lo halves of the chunk go to 16-byte chunks 2ch + 4, 2ch + 5 of the row
+        const uint32_t a_off2 = (uint32_t)r0 * 128u + (uint32_t)(((2 * ch + 4) ^ (r0 & 7)) << 4);
+        const uint32_t a_off3 = (uint32_t)r0 * 128u + (uint32_t)(((2 * ch + 5) ^ (r0 & 7)) << 4);
         // epilogue duty: warps 0..3 drain rows 0..127 of a tile, warps 8..11 rows 128..255 (TMEM lane quarter = warp % 4)
         const bool is_epi = (warp & 7) < 4;
         int ep_done = 0, prod_done = 0;
@@ -319,7 +377,7 @@ dcn_tc_split_kernel(const __grid_constant__ CUtensorMap mapW, const float* __res
             const int g_slot = kb & (S_NTAB - 1);
             const uint32_t g_phase = (uint32_t)(kb / S_NTAB) & 1u;
             poll_epilogue();
-            const float* xs = xt + (c_slab * TBK + ch * 8);
+            const float* xs = xt + (c_slab * SLAB + ch * 8);
             const int* tb = tab_base + g_slot * tab_n + gsub * TAB_STRIDE + r0;
             const float* tw = tab_w + g_slot * 4 * tab_n + gsub * TAB_STRIDE + r0;
             wait_poll(&tab_full[g_slot], g_phase);
@@ -327,14 +385,15 @@ dcn_tc_split_kernel(const __grid_constant__ CUtensorMap mapW, const float* __res
             uint8_t* A = smem + (size_t)stage * prm.stage_bytes;
             if (tg == 0) {        // weight tile of this K step (TMA, lands on the same full barrier)
                 mbar_expect_tx(&full[stage], Co * 128);
-                tma_load_3d(A + T_A_BYTES, &mapW, &full[stage], c_tap * C + c_slab * TBK, 0, 0);
+                // (X3: a tap's packed row is 2C floats, one 32-float block per 16-channel slab)
+                tma_load_3d(A + T_A_BYTES, &mapW, &full[stage], c_tap * (X3 ? 2 * C : C) + c_slab * TBK, 0, 0);
             }
 #pragma unroll 1
-            for (int pr = 0; pr < 2; ++pr) {
+            for (int pr = 0; pr < ITEMS / 2; ++pr) {
 #pragma unroll
                 for (int ii = 0; ii < 2; ++ii) {
                     const int i = pr * 2 + ii;
-                    const int r = 64 * i;
+                    const int r = RSTEP * i;
                     const int bf = tb[r];
                     const float w0 = tw[r], w1 = tw[r + tab_n], w2 = tw[r + 2 * tab_n], w3 = tw[r + 3 * tab_n];
                     const unsigned i0 = (unsigned)(bf & ~3);
@@ -344,17 +403,28 @@ dcn_tc_split_kernel(const __grid_constant__ CUtensorMap mapW, const float* __res
                     const F8 v0 = ldg8(xs + i0), v1 = ldg8(xs + i1), v2 = ldg8(xs + i2), v3 = ldg8(xs + i3);
                     const float2 p0 = make_float2(w0, w0), p1 = make_float2(w1, w1), p2 = make_float2(w2, w2),
                                  p3 = make_float2(w3, w3);
-                    float2 o[4];
+                    float2 o[4], ol[4];
 #pragma unroll
                     for (int e = 0; e < 4; ++e) {
                         float2 a = __fmul2_rn(p0, v0.v[e]);
                         a = __ffma2_rn(p1, v1.v[e], a);
                         a = __ffma2_rn(p2, v2.v[e], a);
                         a = __ffma2_rn(p3, v3.v[e], a);
-                        o[e] = make_float2(tf32_round_bits(a.x), tf32_round_bits(a.y));
+                        if (X3) {
+                            tf32_split_bits(a.x, o[e].x, ol[e].x);
+                            tf32_split_bits(a.y, o[e].y, ol[e].y);
+                        } else {
+                            o[e] = make_float2(tf32_round_bits(a.x), tf32_round_bits(a.y));
+                        }
                     }
-                    *reinterpret_cast<float4*>(A + a_off0 + i * (64 * 128)) = make_float4(o[0].x, o[0].y, o[1].x, o[1].y);
-                    *reinterpret_cast<float4*>(A + a_off1 + i * (64 * 128)) = make_float4(o[2].x, o[2].y, o[3].x, o[3].y);
+                    *reinterpret_cast<float4*>(A + a_off0 + i * (RSTEP * 128)) = make_float4(o[0].x, o[0].y, o[1].x, o[1].y);
+                    *reinterpret_cast<float4*>(A + a_off1 + i * (RSTEP * 128)) = make_float4(o[2].x, o[2].y, o[3].x, o[3].y);
+                    if (X3) {
+                        *reinterpret_cast<float4*>(A + a_off2 + i * (RSTEP * 128)) =
+                            make_float4(ol[0].x, ol[0].y, ol[1].x, ol[1].y);
+                        *reinterpret_cast<float4*>(A + a_off3 + i * (RSTEP * 128)) =
+                            make_float4(ol[2].x, ol[2].y, ol[3].x, ol[3].y);
+                    }
                 }
             }
             fence_proxy_async();
@@ -461,7 +531,8 @@ dcn_tc_split_kernel(const __grid_constant__ CUtensorMap mapW, const float* __res
                     l_tile += gridDim.x;
                     if (l_kb + 1 < total_kb) decode_rows(l_tile);
                 }
-                l_dg0 = (prm.cdg >= TBK) ? (l_slab * TBK) / prm.cdg : l_slab * (TBK / prm.cdg);
+                constexpr int SLAB = X3 ? TBK_X3 : TBK;
+                l_dg0 = (prm.cdg >= SLAB) ? (l_slab * SLAB) / prm.cdg : l_slab * (SLAB / prm.cdg);
             }
         };
         int d_tap = 0;                                           // tap of the table being decoded
@@ -557,7 +628,7 @@ dcn_tc_split_kernel(const __grid_constant__ CUtensorMap mapW, const float* __res
         }
     } else {
         // ------------------------------------------------------------------ MMA issuer
-        if (lane == 0) dcn_mma_issuer(prm, smem, full, empty, tfull, tempty, tmem_base, nkb_tile);
+        if (lane == 0) dcn_mma_issuer<X3>(prm, smem, full, empty, tfull, tempty, tmem_base, nkb_tile);
         __syncwarp();
     }
     tc_fence_before();
@@ -568,16 +639,23 @@ dcn_tc_split_kernel(const __grid_constant__ CUtensorMap mapW, const float* __res
     }
 }
 
-int dcn_pack_weights(const float* w, float* wt, int Co, int C, int K, cudaStream_t st) {
-    dcn_weight_repack_kernel<<<cdiv(Co * C * K, 256), 256, 0, st>>>(w, wt, Co, C, K);
+int dcn_pack_weights(const float* w, float* wt, int Co, int C, int K, cudaStream_t st, bool x3) {
+    if (x3) {
+        MREFSR_CHECK(C % TBK_X3 == 0, ERR_BAD_ARG, "pack_weights (x3): C %% 16 != 0 (C = %d)", C);
+        dcn_weight_repack_x3_kernel<<<cdiv(Co * C * K, 256), 256, 0, st>>>(w, wt, Co, C, K);
+    } else {
+        dcn_weight_repack_kernel<<<cdiv(Co * C * K, 256), 256, 0, st>>>(w, wt, Co, C, K);
+    }
     MREFSR_LAUNCH_CHECK();
     count_launches(1);
     return 0;
 }
 
-int dcn_nchw_to_nhwc(const float* x, float* xt, int B, int C, int HW, cudaStream_t st, bool round_tf32) {
-    if (round_tf32) nchw_to_nhwc_kernel<true><<<dim3(cdiv(HW, 32), cdiv(C, 128), B), 256, 0, st>>>(x, xt, C, HW);
-    else nchw_to_nhwc_kernel<false><<<dim3(cdiv(HW, 32), cdiv(C, 128), B), 256, 0, st>>>(x, xt, C, HW);
+int dcn_nchw_to_nhwc(const float* x, float* xt, int B, int C, int HW, cudaStream_t st, bool round_tf32, float* xt_lo) {
+    const dim3 grid(cdiv(HW, 32), cdiv(C, 128), B);
+    if (xt_lo) nchw_to_nhwc_kernel<true, true><<<grid, 256, 0, st>>>(x, xt, C, HW, xt_lo);
+    else if (round_tf32) nchw_to_nhwc_kernel<true><<<grid, 256, 0, st>>>(x, xt, C, HW, nullptr);
+    else nchw_to_nhwc_kernel<false><<<grid, 256, 0, st>>>(x, xt, C, HW, nullptr);
     MREFSR_LAUNCH_CHECK();
     count_launches(1);
     return 0;
@@ -594,7 +672,8 @@ bool dcn_tc_eligible(const DcnShape& s) {
 
 size_t dcn_tc_workspace_bytes(const DcnShape& s, int mode) {
     if (mode == MREFSR_DCN_FP32 || !dcn_tc_eligible(s)) return 0;
-    return align_up((size_t)s.B * s.C * s.H * s.W * 4, 1024) + align_up((size_t)s.Co * s.C * s.kh * s.kw * 4, 1024);
+    const size_t wfloats = (size_t)s.Co * s.C * s.kh * s.kw * (mode == MREFSR_DCN_TF32X3 ? 2 : 1);   // X3: hi + lo
+    return align_up((size_t)s.B * s.C * s.H * s.W * 4, 1024) + align_up(wfloats * 4, 1024);
 }
 
 // Row -> position mapping of the CTA tiles for prm.s (fills tiles, tile2d and the patch geometry)
@@ -669,7 +748,8 @@ int dcn_forward_tc_impl(const float* x, const float* w, const float* bias, const
                         const long long* max_idx, int flow_scale, float* out, const DcnShape& s, void* workspace,
                         size_t workspace_bytes, cudaStream_t st, int layout_flags, float out_slope,
                         const DcnOutputs* multi) {
-    const size_t need = dcn_tc_workspace_bytes(s, MREFSR_DCN_TF32);
+    const bool x3 = (layout_flags & MREFSR_DCN_X3) != 0;
+    const size_t need = dcn_tc_workspace_bytes(s, x3 ? MREFSR_DCN_TF32X3 : MREFSR_DCN_TF32);
     MREFSR_CHECK(workspace && workspace_bytes >= need, ERR_WORKSPACE, "dcn forward: workspace too small (%zu < %zu)",
                  workspace_bytes, need);
     MREFSR_CHECK((reinterpret_cast<uintptr_t>(workspace) & 1023) == 0, ERR_WORKSPACE,
@@ -683,30 +763,31 @@ int dcn_forward_tc_impl(const float* x, const float* w, const float* bias, const
             MREFSR_CHECK((reinterpret_cast<uintptr_t>(x) & 31) == 0, ERR_BAD_ARG, "dcn forward: NHWC input must be 32-byte aligned");
             xt = const_cast<float*>(x);
         } else {
-            nchw_to_nhwc_kernel<false><<<dim3(cdiv(HW, 32), cdiv(s.C, 128), s.B), 256, 0, st>>>(x, xt, s.C, HW);
+            nchw_to_nhwc_kernel<false><<<dim3(cdiv(HW, 32), cdiv(s.C, 128), s.B), 256, 0, st>>>(x, xt, s.C, HW, nullptr);
             MREFSR_LAUNCH_CHECK();
             count_launches(1);
         }
-        if (layout_flags & MREFSR_DCN_W_PACKED) {      // packed once by the caller (mrefsr_dcn_pack_weights)
+        if (layout_flags & MREFSR_DCN_W_PACKED) {      // packed once by the caller (mrefsr_dcn_pack_weights[_x3])
             MREFSR_CHECK((reinterpret_cast<uintptr_t>(w) & 15) == 0, ERR_BAD_ARG, "dcn forward: packed weights must be 16-byte aligned");
             wt = const_cast<float*>(w);
         } else {
-            int prc = dcn_pack_weights(w, wt, s.Co, s.C, K, st);
+            int prc = dcn_pack_weights(w, wt, s.Co, s.C, K, st, x3);
             if (prc) return prc;
         }
     }
     CUtensorMap mapW;
-    int rc = make_weight_map(&mapW, wt, s.Co, K * s.C);
+    int rc = make_weight_map(&mapW, wt, s.Co, K * s.C * (x3 ? 2 : 1));
     if (rc) return rc;
     DcnTcParams prm;
     prm.s = s;
     prm.P = s.Ho * s.Wo;
     prm.total_rows = s.B * prm.P;
     dcn_plan_tiles(prm);
-    prm.n_slabs = s.C / TBK;
+    const int slab = x3 ? TBK_X3 : TBK;     // channels per K step (every eligible shape has C % 32 == 0, cdg % 8 == 0)
+    prm.n_slabs = s.C / slab;
     prm.taps = K;
     prm.cdg = s.C / s.DG;
-    prm.gs = prm.cdg >= TBK ? 1 : TBK / prm.cdg;
+    prm.gs = prm.cdg >= slab ? 1 : slab / prm.cdg;
     prm.stage_bytes = T_A_BYTES + s.Co * 128;
     const size_t table_bytes = (size_t)S_NTAB * 5 * prm.gs * (TBM + 4) * 4;
     // stage ring vs L1: at 8 channels per deform group the gather needs the L1 more than a third stage (2.11 vs 1.91 ms
@@ -769,7 +850,10 @@ int dcn_forward_tc_impl(const float* x, const float* w, const float* bias, const
     static const Kernel kernels[2][3] = {   // [FUSED][GS = 1, 2, 4]
         {dcn_tc_split_kernel<false, 1>, dcn_tc_split_kernel<false, 2>, dcn_tc_split_kernel<false, 4>},
         {dcn_tc_split_kernel<true, 1>, dcn_tc_split_kernel<true, 2>, dcn_tc_split_kernel<true, 4>}};
-    const Kernel kern = kernels[prm.fused][prm.gs >> 1];
+    static const Kernel kernels_x3[2][2] = {   // [FUSED][GS = 1, 2]: 16-channel slabs hold at most two deform groups
+        {dcn_tc_split_kernel<false, 1, true>, dcn_tc_split_kernel<false, 2, true>},
+        {dcn_tc_split_kernel<true, 1, true>, dcn_tc_split_kernel<true, 2, true>}};
+    const Kernel kern = x3 ? kernels_x3[prm.fused][prm.gs >> 1] : kernels[prm.fused][prm.gs >> 1];
     ScopedTiming tm(MREFSR_K_DCN_FWD, st);
     MREFSR_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     kern<<<grid, S_THREADS, smem, st>>>(mapW, xt, off, prm.fused ? nullptr : mask, prm.fused ? max_idx : nullptr, bias,
@@ -780,8 +864,9 @@ int dcn_forward_tc_impl(const float* x, const float* w, const float* bias, const
 }
 
 int dcn_forward_tc(const float* x, const float* w, const float* bias, const float* off, const float* mask, float* out,
-                   const DcnShape& s, void* workspace, size_t workspace_bytes, cudaStream_t st) {
-    return dcn_forward_tc_impl(x, w, bias, off, mask, nullptr, 1, out, s, workspace, workspace_bytes, st, 0, 1.f, nullptr);
+                   const DcnShape& s, void* workspace, size_t workspace_bytes, cudaStream_t st, bool x3) {
+    return dcn_forward_tc_impl(x, w, bias, off, mask, nullptr, 1, out, s, workspace, workspace_bytes, st,
+                               x3 ? MREFSR_DCN_X3 : 0, 1.f, nullptr);
 }
 
 }  // namespace mrefsr

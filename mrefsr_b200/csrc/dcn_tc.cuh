@@ -7,6 +7,7 @@ namespace mrefsr {
 
 constexpr int TBM = 256;            // rows (output positions) per CTA tile
 constexpr int TBK = 32;             // fp32 channels per K step (128-byte rows)
+constexpr int TBK_X3 = 16;          // channels per K step of the 3-pass kernels: a 128-byte row is [hi 16 | lo 16]
 constexpr int T_A_BYTES = TBM * 128;
 constexpr int T_SMEM_BUDGET = 150 * 1024;          // stage ring; the rest of the 228 KB stays L1 for the gather
 
@@ -77,6 +78,13 @@ __device__ __forceinline__ long long ldg_early_s64(const long long* p) {
 
 // round-to-nearest (ties away) to tf32 in one integer add: the tensor core ignores the low 13 mantissa bits
 __device__ __forceinline__ float tf32_round_bits(float v) { return __uint_as_float(__float_as_uint(v) + 0x1000u); }
+
+// 3-pass split of v: hi = v rounded to tf32 with the low bits CLEARED (v - hi must be the exact remainder, so hi cannot
+// rely on the tensor core's truncation), lo = the remainder rounded like tf32_round_bits.  hi + lo carries 22 bits.
+__device__ __forceinline__ void tf32_split_bits(float v, float& hi, float& lo) {
+    hi = __uint_as_float((__float_as_uint(v) + 0x1000u) & ~0x1FFFu);
+    lo = tf32_round_bits(v - hi);
+}
 
 // 256-bit read-only load: 8 consecutive channels of one corner (one full 32-byte sector per lane)
 struct F8 {

@@ -14,16 +14,24 @@
 // Persistent CTAs, 128 x 128 output tiles, K step 32 (128-byte rows, SWIZZLE_128B), both operands by TMA (rows / k
 // beyond the matrix are zero-filled by the copy engine, so no tile needs padding in memory), 6-stage ring, two TMEM
 // accumulators so the epilogue of a tile overlaps the MMAs of the next.  Warps: TMA producer, MMA issuer, 4 epilogue.
+//
+// X3 (the backward of the 3-pass DCN mode): each operand comes as a tf32 hi plane and a tf32 lo plane (x = hi + lo); a
+// stage holds four boxes (A hi, B hi, A lo, B lo; 64 KB, so 3 stages) and each 8-wide k step issues lo.hi + hi.lo +
+// hi.hi into the same accumulator: fp32-grade products, the lo.lo term (2^-22 relative) dropped.
 #include "common.cuh"
 #include "../../include/mrefsr_b200.h"
 
 namespace mrefsr {
 
-constexpr int G_BM = 128, G_BN = 128, G_BK = 32, G_STAGES = 6;
-constexpr int G_STAGE_BYTES = (G_BM + G_BN) * 128;
+constexpr int G_BM = 128, G_BN = 128, G_BK = 32;
 constexpr int G_EPI_PITCH = 36;                                    // floats per staged row (32 + 4: conflict-free 16-byte accesses)
 constexpr int G_EPI_BYTES = 4 * 32 * G_EPI_PITCH * 4;              // one 32 x 32 staging tile per epilogue warp
-constexpr int G_SMEM = G_STAGES * G_STAGE_BYTES + 256 + G_EPI_BYTES + 1024;
+template <bool X3> struct GemmGeom {
+    static constexpr int STAGES = X3 ? 3 : 6;
+    static constexpr int STAGE_BYTES = (G_BM + G_BN) * 128 * (X3 ? 2 : 1);
+    static constexpr int SMEM = STAGES * STAGE_BYTES + 256 + G_EPI_BYTES + 1024;
+};
+static_assert(GemmGeom<true>::SMEM <= 227 * 1024, "3-pass ring exceeds shared memory");
 
 struct GemmTcParams {
     int M, N, K;               // per batch item
@@ -37,9 +45,12 @@ struct GemmTcParams {
     int ldd;
 };
 
+template <bool X3>
 __global__ void __launch_bounds__(192, 1)
 gemm_tf32_nt_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ CUtensorMap mapB,
+                    const __grid_constant__ CUtensorMap mapA_lo, const __grid_constant__ CUtensorMap mapB_lo,
                     const GemmTcParams prm) {
+    constexpr int G_STAGES = GemmGeom<X3>::STAGES, G_STAGE_BYTES = GemmGeom<X3>::STAGE_BYTES;
     extern __shared__ __align__(1024) uint8_t smem[];
     if ((smem_u32(smem) & 1023u) != 0u) __trap();
     uint64_t* bars = reinterpret_cast<uint64_t*>(smem + G_STAGES * G_STAGE_BYTES);
@@ -54,6 +65,10 @@ gemm_tf32_nt_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_const
     if (threadIdx.x == 0) {
         tma_prefetch_desc(&mapA);
         tma_prefetch_desc(&mapB);
+        if (X3) {
+            tma_prefetch_desc(&mapA_lo);
+            tma_prefetch_desc(&mapB_lo);
+        }
         for (int s = 0; s < G_STAGES; ++s) {
             mbar_init(&full[s], 1);
             mbar_init(&empty[s], 1);
@@ -104,6 +119,10 @@ gemm_tf32_nt_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_const
                     mbar_expect_tx(&full[stage], G_STAGE_BYTES);
                     tma_load_3d(sa, &mapA, &full[stage], k0, mt * G_BM, prm.a_batched ? z : 0);
                     tma_load_3d(sa + G_BM * 128, &mapB, &full[stage], k0, nt * G_BN, z);
+                    if (X3) {
+                        tma_load_3d(sa + (G_BM + G_BN) * 128, &mapA_lo, &full[stage], k0, mt * G_BM, prm.a_batched ? z : 0);
+                        tma_load_3d(sa + (2 * G_BM + G_BN) * 128, &mapB_lo, &full[stage], k0, nt * G_BN, z);
+                    }
                     if (++stage == G_STAGES) {
                         stage = 0;
                         phase ^= 1;
@@ -134,7 +153,15 @@ gemm_tf32_nt_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_const
                     const uint32_t sb = sa + G_BM * 128;
 #pragma unroll
                     for (int kk = 0; kk < 4; ++kk) {
-                        umma_tf32(tacc, umma_desc_sw128(sa + kk * 32, 0), umma_desc_sw128(sb + kk * 32, 0), idesc, accumulate);
+                        const uint64_t ah = umma_desc_sw128(sa + kk * 32, 0), bh = umma_desc_sw128(sb + kk * 32, 0);
+                        if (X3) {
+                            const uint32_t sal = sa + (G_BM + G_BN) * 128, sbl = sal + G_BM * 128;
+                            umma_tf32(tacc, umma_desc_sw128(sal + kk * 32, 0), bh, idesc, accumulate);
+                            umma_tf32(tacc, ah, umma_desc_sw128(sbl + kk * 32, 0), idesc, 1);
+                            umma_tf32(tacc, ah, bh, idesc, 1);
+                        } else {
+                            umma_tf32(tacc, ah, bh, idesc, accumulate);
+                        }
                         accumulate = 1;
                     }
                     umma_commit(&empty[stage]);
@@ -223,22 +250,43 @@ bool gemm_tc_operands_ok(const void* A, int lda, long long a_batch_stride, const
 
 // D[o] (M x N, row pitch ldd, outputs d_stride elements apart) = A . B^T as described in the file header.
 // a_batch_stride == 0: A shared by all batch items.  reduce != 0: `splits` partial outputs (see header).
+// A_lo / B_lo (both or neither): the 3-pass variant, A / B are then the hi planes.
 int gemm_tf32_nt(const float* A, int lda, long long a_batch_stride, const float* B, int ldb, long long b_batch_stride,
                  float* D, int ldd, long long d_stride, int M, int N, int K, int batch, int reduce, int splits,
-                 cudaStream_t st) {
+                 cudaStream_t st, const float* A_lo, const float* B_lo) {
     MREFSR_CHECK(M > 0 && N > 0 && K > 0 && batch > 0, ERR_BAD_ARG, "gemm: bad sizes");
     MREFSR_CHECK(gemm_tc_operands_ok(A, lda, a_batch_stride, B, ldb, b_batch_stride), ERR_BAD_ARG,
                  "gemm: operands must be 16-byte aligned with row pitches that are multiples of 4 floats");
-    CUtensorMap mapA, mapB;
+    const bool x3 = A_lo != nullptr;
+    MREFSR_CHECK((B_lo != nullptr) == x3, ERR_BAD_ARG, "gemm: the 3-pass variant needs both lo planes");
+    MREFSR_CHECK(!x3 || gemm_tc_operands_ok(A_lo, lda, a_batch_stride, B_lo, ldb, b_batch_stride), ERR_BAD_ARG,
+                 "gemm: lo planes must be 16-byte aligned");
     const bool a_batched = a_batch_stride != 0;
-    int rc = make_tensor_map_3d_strided(&mapA, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, A, (uint64_t)K, (uint64_t)M,
-                                        a_batched ? (uint64_t)batch : 1, (uint64_t)lda * 4,
-                                        (uint64_t)(a_batched ? a_batch_stride : (long long)lda * M) * 4, G_BK, G_BM,
-                                        CU_TENSOR_MAP_SWIZZLE_128B);
+    auto map_a = [&](CUtensorMap* map, const float* a) {
+        return make_tensor_map_3d_strided(map, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, a, (uint64_t)K, (uint64_t)M,
+                                          a_batched ? (uint64_t)batch : 1, (uint64_t)lda * 4,
+                                          (uint64_t)(a_batched ? a_batch_stride : (long long)lda * M) * 4, G_BK, G_BM,
+                                          CU_TENSOR_MAP_SWIZZLE_128B);
+    };
+    auto map_b = [&](CUtensorMap* map, const float* b) {
+        return make_tensor_map_3d_strided(map, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, b, (uint64_t)K, (uint64_t)N,
+                                          (uint64_t)batch, (uint64_t)ldb * 4, (uint64_t)b_batch_stride * 4, G_BK, G_BN,
+                                          CU_TENSOR_MAP_SWIZZLE_128B);
+    };
+    CUtensorMap mapA, mapB, mapA_lo, mapB_lo;
+    int rc = map_a(&mapA, A);
     if (rc) return rc;
-    rc = make_tensor_map_3d_strided(&mapB, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, B, (uint64_t)K, (uint64_t)N, (uint64_t)batch,
-                                    (uint64_t)ldb * 4, (uint64_t)b_batch_stride * 4, G_BK, G_BN, CU_TENSOR_MAP_SWIZZLE_128B);
+    rc = map_b(&mapB, B);
     if (rc) return rc;
+    if (x3) {
+        rc = map_a(&mapA_lo, A_lo);
+        if (rc) return rc;
+        rc = map_b(&mapB_lo, B_lo);
+        if (rc) return rc;
+    } else {
+        mapA_lo = mapA;      // unused by the one-pass kernel
+        mapB_lo = mapB;
+    }
     GemmTcParams prm;
     prm.M = M;
     prm.N = N;
@@ -256,8 +304,15 @@ int gemm_tf32_nt(const float* A, int lda, long long a_batch_stride, const float*
     const long long items = (long long)(reduce ? splits : batch) * prm.m_tiles * prm.n_tiles;
     int grid = sm_count();
     if (grid > items) grid = (int)items;
-    MREFSR_CUDA(cudaFuncSetAttribute(gemm_tf32_nt_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, G_SMEM));
-    gemm_tf32_nt_kernel<<<grid, 192, G_SMEM, st>>>(mapA, mapB, prm);
+    if (x3) {
+        MREFSR_CUDA(cudaFuncSetAttribute(gemm_tf32_nt_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                         GemmGeom<true>::SMEM));
+        gemm_tf32_nt_kernel<true><<<grid, 192, GemmGeom<true>::SMEM, st>>>(mapA, mapB, mapA_lo, mapB_lo, prm);
+    } else {
+        MREFSR_CUDA(cudaFuncSetAttribute(gemm_tf32_nt_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                         GemmGeom<false>::SMEM));
+        gemm_tf32_nt_kernel<false><<<grid, 192, GemmGeom<false>::SMEM, st>>>(mapA, mapB, mapA_lo, mapB_lo, prm);
+    }
     MREFSR_LAUNCH_CHECK();
     count_launches(1);
     return 0;

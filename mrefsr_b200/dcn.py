@@ -20,30 +20,41 @@ from torch.nn.modules.utils import _pair, _single
 
 from . import _lib
 
-DCN_AUTO, DCN_FP32, DCN_TF32 = 0, 1, 2
-_MODES = {'auto': DCN_AUTO, 'fp32': DCN_FP32, 'tf32': DCN_TF32}
+DCN_AUTO, DCN_FP32, DCN_TF32, DCN_TF32X3 = 0, 1, 2, 3
+_MODES = {'auto': DCN_AUTO, 'fp32': DCN_FP32, 'tf32': DCN_TF32, 'tf32x3': DCN_TF32X3}
 _default_mode = DCN_AUTO
+_FLAG_X3 = 8          # MREFSR_DCN_X3: layout flag of the fused DynAgg entry points
+
+
+def _mode(mode):
+    return _default_mode if mode is None else (_MODES[mode] if isinstance(mode, str) else int(mode))
 
 
 def set_default_mode(mode):
-    """'auto' | 'fp32' (exact, CUDA cores) | 'tf32' (tcgen05)."""
+    """'auto' | 'fp32' (exact, CUDA cores) | 'tf32' (tcgen05) | 'tf32x3' (tcgen05 with 3-pass split-tf32 operands:
+    fp32-grade results in the forward and in the backward GEMMs, same shapes as 'tf32', and the fused DynAgg entry
+    points follow it too)."""
     global _default_mode
-    _default_mode = _MODES[mode] if isinstance(mode, str) else int(mode)
+    _default_mode = _mode(mode)
 
 
-def pack_weight(weight):
+def pack_weight(weight, mode=None):
     """tf32-rounded [Co][tap][C] copy of a DCN weight, the B operand of the tcgen05 kernels (mrefsr_dcn_pack_weights).
+    mode (default: the default mode) 'tf32x3': the 3-pass kernels' hi / lo packing [Co][tap][C/16][hi 16 | lo 16]
+    (mrefsr_dcn_pack_weights_x3, twice the size), the one `dynagg_dcn_forward` wants while the default mode is 'tf32x3'.
     The forward entry points repack on every call (a few microseconds); a caller whose weights are frozen may pack once
     and hand the result to `dynagg_dcn_forward(..., weight_packed=...)`.  There is deliberately NO implicit cache:
     torch's version counter does not see `weight.data.copy_(...)`-style updates, and a stale packing would be a silent
     wrong answer for a 0.2 % gain."""
     _lib.require_cuda(weight)
+    x3 = _mode(mode) == DCN_TF32X3
     w = weight.detach().contiguous().float()
     co, c, kh, kw = w.shape
-    packed = torch.empty(co, kh * kw * c, dtype=torch.float32, device=w.device)
+    packed = torch.empty(co, kh * kw * c * (2 if x3 else 1), dtype=torch.float32, device=w.device)
+    fn = 'mrefsr_dcn_pack_weights_x3' if x3 else 'mrefsr_dcn_pack_weights'
     with torch.cuda.device(w.device):
-        rc = _lib.lib().mrefsr_dcn_pack_weights(_lib.ptr(w), _lib.ptr(packed), co, c, kh * kw, _lib.stream_ptr(w.device))
-    _lib.check(rc, 'mrefsr_dcn_pack_weights')
+        rc = getattr(_lib.lib(), fn)(_lib.ptr(w), _lib.ptr(packed), co, c, kh * kw, _lib.stream_ptr(w.device))
+    _lib.check(rc, fn)
     return packed
 
 
@@ -65,13 +76,14 @@ def _check_shapes(input, offset, mask, weight, groups, dg, ho, wo):
 
 
 def dcn_forward_raw(input, offset, mask, weight, bias, stride, padding, dilation, groups, dg, mode=None):
-    """Forward on contiguous fp32 CUDA tensors -> output [B,Co,Ho,Wo] (no autograd).  mask=None: all-ones (DCNv1)."""
+    """Forward on contiguous fp32 CUDA tensors -> output [B,Co,Ho,Wo] (no autograd).  mask=None: all-ones (DCNv1).
+    mode: 'auto' | 'fp32' | 'tf32' | 'tf32x3' (or the C enum value); None: the default mode."""
     lib = _lib.lib()
     b, c, h, w = input.shape
     co, _, kh, kw = weight.shape
     ho, wo = _out_hw(h, w, kh, kw, stride, padding, dilation)
     _check_shapes(input, offset, mask, weight, groups, dg, ho, wo)
-    m = _default_mode if mode is None else (_MODES[mode] if isinstance(mode, str) else int(mode))
+    m = _mode(mode)
     out = torch.empty(b, co, ho, wo, dtype=torch.float32, device=input.device)
     with torch.cuda.device(input.device):
         nbytes = lib.mrefsr_dcn_workspace_bytes(b, c, h, w, co, kh, kw, stride[0], stride[1], padding[0], padding[1],
@@ -115,8 +127,11 @@ def dynagg_dcn_forward_into(input, conv_out, max_idx, flow_scale, weight, bias, 
     if not 1 <= len(out_ptrs) <= 8:
         raise ValueError('1..8 destination buffers')
     arr = (ctypes.c_void_p * len(out_ptrs))(*[int(p) for p in out_ptrs])
+    x3 = _default_mode == DCN_TF32X3
+    flags = (1 if in_cl else 0) | (_FLAG_X3 if x3 else 0)
     with torch.cuda.device(x.device):
-        nbytes = lib.mrefsr_dcn_workspace_bytes(b, c, h, w, co, 3, 3, 1, 1, 1, 1, 1, 1, 1, dg, DCN_TF32, 0)
+        nbytes = lib.mrefsr_dcn_workspace_bytes(b, c, h, w, co, 3, 3, 1, 1, 1, 1, 1, 1, 1, dg,
+                                                DCN_TF32X3 if x3 else DCN_TF32, 0)
         ws, ws_bytes = _lib.workspace(nbytes, x.device)
         if slab_rows:
             if slab_rows * len(out_ptrs) < h:
@@ -124,13 +139,13 @@ def dynagg_dcn_forward_into(input, conv_out, max_idx, flow_scale, weight, bias, 
             rc = lib.mrefsr_dynagg_dcn_forward_slabs(_lib.ptr(x), _lib.ptr(wgt), _lib.ptr(bs), _lib.ptr(co_), _lib.ptr(mi),
                                                      int(flow_scale), ctypes.cast(arr, ctypes.c_void_p), len(out_ptrs),
                                                      int(slab_rows), int(dst_group), int(dst_stride), int(dst_offset), b, c,
-                                                     h, w, co, dg, int(bs is not None), 1 if in_cl else 0, float(out_slope),
+                                                     h, w, co, dg, int(bs is not None), flags, float(out_slope),
                                                      ws, ws_bytes, _lib.stream_ptr(x.device))
         else:
             rc = lib.mrefsr_dynagg_dcn_forward_multi(_lib.ptr(x), _lib.ptr(wgt), _lib.ptr(bs), _lib.ptr(co_), _lib.ptr(mi),
                                                      int(flow_scale), ctypes.cast(arr, ctypes.c_void_p), len(out_ptrs),
                                                      int(dst_group), int(dst_stride), int(dst_offset), b, c, h, w, co, dg,
-                                                     int(bs is not None), 1 if in_cl else 0, float(out_slope), ws, ws_bytes,
+                                                     int(bs is not None), flags, float(out_slope), ws, ws_bytes,
                                                      _lib.stream_ptr(x.device))
     _lib.check(rc, 'mrefsr_dynagg_dcn_forward_slabs' if slab_rows else 'mrefsr_dynagg_dcn_forward_multi')
 
@@ -143,7 +158,9 @@ def dynagg_dcn_forward(input, conv_out, max_idx, flow_scale, weight, bias, defor
     input [B,C,H,W], conv_out [B,3*dg*9,H,W], max_idx int64 [B,H/s-2,W/s-2] -> [B,Co,H,W].
     A torch.channels_last `input` is consumed as it is (it already is the gather layout); the result is
     channels_last when `out_channels_last` (default: follows the input).  out_slope: leaky-ReLU slope applied to the
-    result in the epilogue (1.0 = none).  weight_packed: optional `pack_weight(weight)` (skips the per-call repack)."""
+    result in the epilogue (1.0 = none).  weight_packed: optional `pack_weight(weight)` (skips the per-call repack).
+    While the default mode is 'tf32x3' this runs the 3-pass kernel (fp32-grade) and weight_packed must come from
+    `pack_weight(weight, 'tf32x3')`; every other mode runs the tf32 kernel, as this entry point always has."""
     _lib.require_cuda(input, conv_out, max_idx, weight, bias)
     lib = _lib.lib()
     x = input.float()
@@ -167,13 +184,16 @@ def dynagg_dcn_forward(input, conv_out, max_idx, flow_scale, weight, bias, defor
         raise RuntimeError('weight shape %s, expected [Co,%d,3,3]' % (tuple(wgt.shape), c))
     out = torch.empty(b, co, h, w, dtype=torch.float32, device=x.device,
                       memory_format=torch.channels_last if out_channels_last else torch.contiguous_format)
-    flags = (1 if in_cl else 0) | (2 if out_channels_last else 0)
+    x3 = _default_mode == DCN_TF32X3
+    flags = (1 if in_cl else 0) | (2 if out_channels_last else 0) | (_FLAG_X3 if x3 else 0)
     if weight_packed is not None:        # pack_weight(weight), made once by a caller whose weights are frozen
-        if tuple(weight_packed.shape) != (co, 9 * c) or weight_packed.dtype != torch.float32 or not weight_packed.is_contiguous():
-            raise RuntimeError('weight_packed must be the result of pack_weight(weight)')
+        if (tuple(weight_packed.shape) != (co, 9 * c * (2 if x3 else 1)) or weight_packed.dtype != torch.float32 or
+                not weight_packed.is_contiguous()):
+            raise RuntimeError('weight_packed must be the result of pack_weight(weight%s)' % (", 'tf32x3'" if x3 else ''))
         wgt, flags = weight_packed, flags | 4
     with torch.cuda.device(x.device):
-        nbytes = lib.mrefsr_dcn_workspace_bytes(b, c, h, w, co, 3, 3, 1, 1, 1, 1, 1, 1, 1, dg, DCN_TF32, 0)
+        nbytes = lib.mrefsr_dcn_workspace_bytes(b, c, h, w, co, 3, 3, 1, 1, 1, 1, 1, 1, 1, dg,
+                                                DCN_TF32X3 if x3 else DCN_TF32, 0)
         ws, ws_bytes = _lib.workspace(nbytes, x.device)
         rc = lib.mrefsr_dynagg_dcn_forward_ex(_lib.ptr(x), _lib.ptr(wgt), _lib.ptr(bs), _lib.ptr(co_), _lib.ptr(mi),
                                               int(flow_scale), _lib.ptr(out), b, c, h, w, co, dg, int(bs is not None),
