@@ -118,6 +118,8 @@ enum {
     MREFSR_DCN_TF32 = 2,
     MREFSR_DCN_TF32X3 = 3,
 };
+/* backward = 0: the scratch of the forward entry points; backward = 1: that of mrefsr_modulated_deform_conv_backward and
+ * of mrefsr_dynagg_dcn_backward (called with 3x3, stride 1, pad 1, dil 1, group 1 and the mode passed to it). */
 MREFSR_API size_t mrefsr_dcn_workspace_bytes(int B, int C, int H, int W, int Co, int kh, int kw, int stride_h, int stride_w,
                                   int pad_h, int pad_w, int dil_h, int dil_w, int group, int deformable_group,
                                   int mode, int backward);
@@ -158,9 +160,9 @@ MREFSR_API int mrefsr_dynagg_offsets(const float* conv_out, const float* pre_off
 MREFSR_API int mrefsr_dynagg_offsets_backward(const float* grad_offset, const float* grad_mask, const float* mask,
                                    float* grad_conv_out, int B, int dg, int K, int H, int W, void* stream);
 
-/* Fused DynAgg forward (inference): DCNv2 whose offsets / masks are assembled inside the gather from the raw
- * conv_offset_mask output and the matcher's arg-max map, so neither the pre-offset tensors nor offset / mask
- * are ever written to HBM:
+/* Fused DynAgg forward: DCNv2 whose offsets / masks are assembled inside the gather from the raw conv_offset_mask
+ * output and the matcher's arg-max map, so neither the pre-offset tensors nor offset / mask are ever written to HBM
+ * (inference; for training, mrefsr_dynagg_dcn_backward below is its backward from the same source):
  *   offset[:, 2(g*9+k)  ] = conv_out[:, 2(g*9+k)  ] + s * flow_y[Y/s - i, X/s - j]      (k = 3i + j)
  *   offset[:, 2(g*9+k)+1] = conv_out[:, 2(g*9+k)+1] + s * flow_x[Y/s - i, X/s - j]
  *   mask = sigmoid(conv_out[:, 2*dg*9 + g*9 + k]),  flow = index_to_flow(max_idx) (0 outside the grid)
@@ -238,6 +240,27 @@ MREFSR_API int mrefsr_dynagg_dcn_forward_slabs(const float* input, const float* 
                                     int dst_offset, int B, int C, int H, int W, int Co, int deformable_group,
                                     int with_bias, int layout_flags, float out_slope, void* workspace,
                                     size_t workspace_bytes, void* stream);
+
+/* Backward of the fused DynAgg forward (training): the gradients of mrefsr_dynagg_dcn_forward_ex's output with respect
+ * to input, weight, bias and the raw conv_offset_mask output, read from the same conv_out + max_idx source.  The
+ * sampling points and masks are computed bit for bit as the forward computes them, and no offset / mask / pre-offset
+ * tensor is materialised:
+ *   grad_conv_out[:, 2(g*9+k)], [:, 2(g*9+k)+1] = d loss / d offset (y, x)   (the flows carry no gradient)
+ *   grad_conv_out[:, 2*dg*9 + g*9 + k]          = d loss / d mask * mask * (1 - mask)
+ * Shapes and requirements as mrefsr_dynagg_dcn_forward (3x3, stride 1, pad 1, dil 1, the tcgen05 shapes, H and W
+ * multiples of flow_scale); grad_output [B, Co, H, W] planes, grad_conv_out [B, 3*dg*9, H, W] planes (overwritten).
+ * grad_input, grad_weight and grad_conv_out may each be NULL (that part is skipped); grad_input is overwritten, in
+ * input's layout; grad_weight / grad_bias are ACCUMULATED into, as in mrefsr_modulated_deform_conv_backward.
+ * layout_flags: MREFSR_DCN_IN_NHWC (input and grad_input are [B, H, W, C]; input 32-byte aligned) or 0.
+ * mode: MREFSR_DCN_TF32 (MREFSR_DCN_AUTO resolves to it) or MREFSR_DCN_TF32X3, the modes the fused forward runs;
+ * MREFSR_DCN_FP32 is refused with ERR_UNSUPPORTED.  workspace: mrefsr_dcn_workspace_bytes(B, C, H, W, Co, 3, 3, 1, 1,
+ * 1, 1, 1, 1, 1, deformable_group, mode, 1), the size of the materialised backward. */
+MREFSR_API int mrefsr_dynagg_dcn_backward(const float* input, const float* weight, const float* conv_out,
+                                          const int64_t* max_idx, int flow_scale, const float* grad_output,
+                                          float* grad_input, float* grad_weight, float* grad_bias, float* grad_conv_out,
+                                          int B, int C, int H, int W, int Co, int deformable_group, int with_bias,
+                                          int layout_flags, int mode, void* workspace, size_t workspace_bytes,
+                                          void* stream);
 
 /* ------------------------------------------------------------------------------------------
  * Trunk glue (SURVEY 8f-2: the plain-convolution network either side of the path; convolutions

@@ -39,6 +39,7 @@ SIGNATURES = {
     'mrefsr_dynagg_dcn_forward_multi': (c_int, [_P] * 5 + [_I] + [_P] + [_I] * 12 + [ctypes.c_float, _P, c_size_t, _P]),
     'mrefsr_dynagg_dcn_forward_slabs': (c_int, [_P] * 5 + [_I] + [_P] + [_I] * 13 + [ctypes.c_float, _P, c_size_t, _P]),
     'mrefsr_dynagg_dcn_forward_ex': (c_int, [_P] * 5 + [_I] + [_P] + [_I] * 8 + [ctypes.c_float, _P, c_size_t, _P]),
+    'mrefsr_dynagg_dcn_backward': (c_int, [_P] * 4 + [_I] + [_P] * 5 + [_I] * 9 + [_P, c_size_t, _P]),
     'mrefsr_dynagg_offsets': (c_int, [_P] * 5 + [_I] * 5 + [_P]),
     'mrefsr_dynagg_offsets_backward': (c_int, [_P] * 4 + [_I] * 5 + [_P]),
     'mrefsr_bias_act': (c_int, [_P, _P, _P, _I, _P, _I, _I, _I, _I, _I, _I, _I, ctypes.c_float, ctypes.c_float, _P]),

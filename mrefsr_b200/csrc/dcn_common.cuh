@@ -10,6 +10,19 @@ struct DcnShape {
 
 __host__ __device__ __forceinline__ int cdiv_d(int a, int b) { return (a + b - 1) / b; }
 
+// Sample sources of the DCN backward kernels: the type of their last argument selects the overload (dcn.cu).
+// PlaneSrc: materialised offset [B, 2*DG*K, Ho, Wo] and mask [B, DG*K, Ho, Wo] planes (the kernels' offset / mask
+// arguments); grad_offset / grad_mask are written as such planes.
+struct PlaneSrc {};
+// DynAggSrc: the fused DynAgg forward's inputs.  The kernels' `offset` argument is the raw conv_offset_mask output
+// [B, 3*DG*K, Ho, Wo] (dy / dx of (g, k) in channels 2(g*K+k) / +1, mask logits in 2*DG*K + g*K + k), flows come from
+// the matcher's arg-max map max_idx [B, hp, wp] at 1/flow_scale resolution, and the gradient with respect to that raw
+// output is written in its layout (`grad_offset` argument).  x_nhwc: the input (and grad_input) is [B, H, W, C].
+struct DynAggSrc {
+    const long long* max_idx;
+    int flow_scale, hp, wp, x_nhwc;
+};
+
 #ifdef __CUDACC__
 // Bilinear sample of one channel plane at fractional (y, x).
 // Rule of deform_conv_cuda_kernel.cu:618 + :468-497: the value is 0 unless -1 < y < H and -1 < x < W; inside,

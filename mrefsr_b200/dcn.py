@@ -152,7 +152,7 @@ def dynagg_dcn_forward_into(input, conv_out, max_idx, flow_scale, weight, bias, 
 
 def dynagg_dcn_forward(input, conv_out, max_idx, flow_scale, weight, bias, deformable_groups, out_slope=1.0,
                        out_channels_last=None, weight_packed=None):
-    """Fused DynAgg forward for inference (no autograd): DCNv2 (3x3, stride 1, pad 1) whose offsets and masks are
+    """Fused DynAgg forward (no autograd; dynagg.DynAggFusedFunction is its autograd node): DCNv2 (3x3, stride 1, pad 1) whose offsets and masks are
     assembled inside the gather from the raw conv_offset_mask output and the matcher's arg-max map
     (ref_mrapa_restoration_arch.py:45-76 + corres_generation_arch.py:30-47, :70-105 for one scale).
     input [B,C,H,W], conv_out [B,3*dg*9,H,W], max_idx int64 [B,H/s-2,W/s-2] -> [B,Co,H,W].
@@ -200,6 +200,47 @@ def dynagg_dcn_forward(input, conv_out, max_idx, flow_scale, weight, bias, defor
                                               flags, float(out_slope), ws, ws_bytes, _lib.stream_ptr(x.device))
     _lib.check(rc, 'mrefsr_dynagg_dcn_forward_ex')
     return out
+
+
+def dynagg_dcn_backward_raw(input, conv_out, max_idx, flow_scale, weight, grad_output, deformable_groups, with_bias,
+                            need_input=True, need_conv=True, need_weight=True, mode=None):
+    """Backward of `dynagg_dcn_forward` (mrefsr_dynagg_dcn_backward, no autograd) -> (grad_input, grad_conv_out,
+    grad_weight, grad_bias); parts not requested (or no bias) are None.  input: the fp32 tensor the forward read (dense
+    NCHW or channels_last; grad_input comes back in the same layout); conv_out fp32 NCHW [B,3*dg*9,H,W]; max_idx int64
+    [B,H/s-2,W/s-2]; weight fp32 [Co,C,3,3]; grad_output fp32 NCHW [B,Co,H,W].  grad_conv_out = [d offset,
+    d mask * mask * (1 - mask)] at conv_out's channels.  mode None: 'tf32x3' while that is the default mode, else 'tf32'
+    (the modes the fused forward runs); 'fp32' is refused."""
+    from .trunk import is_channels_last
+    lib = _lib.lib()
+    in_cl = is_channels_last(input)
+    b, c, h, w = input.shape
+    co, dg = weight.shape[0], deformable_groups
+    m = (DCN_TF32X3 if _default_mode == DCN_TF32X3 else DCN_TF32) if mode is None else _mode(mode)
+    for name, t in (('input', input), ('conv_out', conv_out), ('weight', weight), ('grad_output', grad_output)):
+        if t.dtype != torch.float32 or not (t.is_contiguous() or (t is input and in_cl)):
+            raise RuntimeError('%s must be a dense fp32 tensor' % name)
+    if tuple(conv_out.shape) != (b, 3 * dg * 9, h, w) or tuple(grad_output.shape) != (b, co, h, w):
+        raise RuntimeError('conv_out / grad_output shapes %s / %s, expected %s / %s' % (
+            tuple(conv_out.shape), tuple(grad_output.shape), (b, 3 * dg * 9, h, w), (b, co, h, w)))
+    if max_idx.dtype != torch.int64 or not max_idx.is_contiguous() or \
+            tuple(max_idx.shape) != (b, h // flow_scale - 2, w // flow_scale - 2):
+        raise RuntimeError('max_idx must be contiguous int64 [%d,%d,%d]' % (b, h // flow_scale - 2, w // flow_scale - 2))
+    if tuple(weight.shape[1:]) != (c, 3, 3):
+        raise RuntimeError('weight shape %s, expected [Co,%d,3,3]' % (tuple(weight.shape), c))
+    gi = torch.empty_like(input) if need_input else None
+    gc = torch.empty_like(conv_out) if need_conv else None
+    gw = torch.zeros_like(weight) if need_weight else None
+    gb = torch.zeros(co, dtype=torch.float32, device=input.device) if with_bias else None
+    with torch.cuda.device(input.device):
+        nbytes = lib.mrefsr_dcn_workspace_bytes(b, c, h, w, co, 3, 3, 1, 1, 1, 1, 1, 1, 1, dg,
+                                                DCN_TF32 if m == DCN_AUTO else m, 1)
+        ws, ws_bytes = _lib.workspace(nbytes, input.device)
+        rc = lib.mrefsr_dynagg_dcn_backward(_lib.ptr(input), _lib.ptr(weight), _lib.ptr(conv_out), _lib.ptr(max_idx),
+                                            int(flow_scale), _lib.ptr(grad_output), _lib.ptr(gi), _lib.ptr(gw),
+                                            _lib.ptr(gb), _lib.ptr(gc), b, c, h, w, co, dg, int(with_bias),
+                                            1 if in_cl else 0, m, ws, ws_bytes, _lib.stream_ptr(input.device))
+    _lib.check(rc, 'mrefsr_dynagg_dcn_backward')
+    return gi, gc, gw, gb
 
 
 def _nchw(t):

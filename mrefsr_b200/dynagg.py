@@ -5,6 +5,8 @@ Drop-in for basicsr.archs.ref_mrapa_restoration_arch.DynAgg (:11-76): same const
 zeros_like / strided scatter / add / sigmoid sequence (:55-68) is one kernel, and the reference's host-syncing
 ``if offset_mean > 100`` check (:69-73, which also references an undefined ``logger``) is replaced by an
 asynchronous device-side accumulator readable through ``last_offset_abs_mean()``.
+``forward_fused(x, max_idx, flow_scale)`` takes the matcher's arg-max map instead of pre-offsets and builds offsets
+and masks inside the DCN gather, in the forward and (DynAggFusedFunction) in the backward.
 """
 import torch
 from torch import nn
@@ -131,6 +133,64 @@ class DynAggDCNFunction(Function):
                 gb if ctx.with_bias and ctx.needs_input_grad[4] else None, None, None, None, None)
 
 
+class DynAggFusedFunction(Function):
+    """Training path of DynAgg.forward_fused as ONE autograd node: (x, conv_out, max_idx, weight, bias) -> DCNv2 output.
+
+    The forward is the launch `dcn.dynagg_dcn_forward` makes (offsets / masks assembled inside the gather from the raw
+    conv_offset_mask output and the matcher's arg-max map); the backward reads the same source
+    (mrefsr_dynagg_dcn_backward), so neither pass writes pre-offset, offset or mask tensors, and the gradient of
+    conv_out comes straight out of the coordinate kernel.  out_slope / out_like_conv as in DynAggDCNFunction."""
+
+    @staticmethod
+    def forward(ctx, x, conv_out, max_idx, flow_scale, weight, bias, dg, out_slope=1.0, out_like_conv=False):
+        from .dcn import dynagg_dcn_forward, _nchw
+        from .trunk import from_nchw_f32, is_channels_last
+        _lib.require_cuda(x, conv_out, max_idx, weight, bias)
+        ctx.conv_dtype, ctx.x_dtype, ctx.w_dtype = conv_out.dtype, x.dtype, weight.dtype
+        ctx.conv_cl = is_channels_last(conv_out)
+        ctx.with_bias, ctx.dg, ctx.flow_scale = bias is not None, dg, int(flow_scale)
+        x32 = x.float()
+        if not is_channels_last(x32):
+            x32 = x32.contiguous()
+        co, wgt, mi = _nchw(conv_out), weight.contiguous().float(), max_idx.contiguous()
+        out = dynagg_dcn_forward(x32, co, mi, flow_scale, wgt, bias, dg, out_channels_last=False)
+        ctx.out_slope = float(out_slope)
+        if out_like_conv:
+            res = from_nchw_f32(out, conv_out.dtype, ctx.conv_cl, slope=ctx.out_slope)
+        else:
+            if ctx.out_slope != 1.0:
+                out = torch.nn.functional.leaky_relu_(out, ctx.out_slope)
+            res = out.to(x.dtype)
+        if ctx.out_slope != 1.0:
+            ctx.save_for_backward(x32, co, mi, wgt, res)
+        else:
+            ctx.save_for_backward(x32, co, mi, wgt)
+        return res
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, grad_output):
+        from .dcn import dynagg_dcn_backward_raw, _nchw
+        from .trunk import from_nchw_f32, to_nchw_f32
+        if ctx.out_slope != 1.0:
+            x32, co, mi, wgt, res = ctx.saved_tensors
+            if grad_output.dtype != res.dtype:
+                grad_output = grad_output.to(res.dtype)
+            g32 = to_nchw_f32(grad_output, gate=res, slope=ctx.out_slope)
+        else:
+            x32, co, mi, wgt = ctx.saved_tensors
+            g32 = _nchw(grad_output)
+        gi, g_conv, gw, gb = dynagg_dcn_backward_raw(x32, co, mi, ctx.flow_scale, wgt, g32, ctx.dg, ctx.with_bias,
+                                                     need_input=ctx.needs_input_grad[0],
+                                                     need_conv=ctx.needs_input_grad[1],
+                                                     need_weight=ctx.needs_input_grad[4])
+        if g_conv is not None and (ctx.conv_cl or ctx.conv_dtype != torch.float32):
+            g_conv = from_nchw_f32(g_conv, ctx.conv_dtype, ctx.conv_cl)
+        cast = (lambda t, dt: None if t is None else t.to(dt))
+        return (cast(gi, ctx.x_dtype), g_conv, None, None, cast(gw, ctx.w_dtype),
+                gb if ctx.with_bias and ctx.needs_input_grad[5] else None, None, None, None)
+
+
 class DynAgg(ModulatedDeformConv2d):
 
     def __init__(self, in_channels, out_channels, kernel_size, stride, padding, dilation=1, groups=1,
@@ -155,9 +215,12 @@ class DynAgg(ModulatedDeformConv2d):
             return None
         return float(self._stats.item()) / self._stats_count
 
-    def forward_fused(self, x, max_idx, flow_scale, out_slope=1.0):
-        """Inference fast path (no autograd): same result as forward(x, pre_offset) where pre_offset is the
-        matcher's shifted flow at this scale, but offsets / masks / pre-offsets never touch HBM."""
+    def forward_fused(self, x, max_idx, flow_scale, out_slope=1.0, out_like_conv=False):
+        """Same result as forward(x, pre_offset) where pre_offset is the matcher's shifted flow at this scale
+        (max_idx int64 [B, H/flow_scale - 2, W/flow_scale - 2]), but offsets / masks / pre-offsets never touch HBM.
+        With grad enabled and x or a parameter requiring grad this is one autograd node (DynAggFusedFunction) whose
+        backward reads the same source; otherwise the inference path.  out_slope: leaky ReLU applied to the result;
+        out_like_conv: the result in the dtype / layout of the offset convolution's output (the trunk's)."""
         from .dcn import dynagg_dcn_forward
         from . import trunk as T
         if not (tuple(self.kernel_size) == (3, 3) and tuple(self.stride) == (1, 1) and tuple(self.padding) == (1, 1)
@@ -168,12 +231,21 @@ class DynAgg(ModulatedDeformConv2d):
         feat = x[1] if self.extra_offset_mask else x
         if self.extra_offset_mask:
             x = x[0]
+        if torch.is_grad_enabled() and (x.requires_grad or feat.requires_grad or
+                                        any(p.requires_grad for p in self.parameters())):
+            out = T.conv_act(feat, self.conv_offset_mask)       # (training: bias add and its gradient fused)
+            return DynAggFusedFunction.apply(x, out, max_idx, flow_scale, self.weight, self.bias, self.deform_groups,
+                                             out_slope, out_like_conv)
         if T.fast_ok(feat):    # the DCN reads planes: bias (+ the NHWC -> NCHW conversion of a channels-last conv) in one pass
             out = T.conv_bias_to_nchw(feat, self.conv_offset_mask)
         else:
             out = self.conv_offset_mask(feat)
-        return dynagg_dcn_forward(x, out, max_idx, flow_scale, self.weight, self.bias, self.deform_groups,
-                                  out_slope=out_slope)
+        y = dynagg_dcn_forward(x, out, max_idx, flow_scale, self.weight, self.bias, self.deform_groups,
+                               out_slope=out_slope)
+        if out_like_conv:      # (the convolution keeps its input's layout; conv_bias_to_nchw hands back planes)
+            y = y.to(dtype=out.dtype, memory_format=torch.channels_last if T.is_channels_last(feat) else
+                     torch.contiguous_format)
+        return y
 
     def forward(self, x, pre_offset, out_slope=1.0, out_like_conv=False):
         """Reference signature forward(x, pre_offset).  out_slope / out_like_conv (fused autograd node only): apply the

@@ -195,11 +195,15 @@ class DynamicAggregationRestoration(nn.Module):
 
     def _forward_stacked(self, x, pres, feats, r):
         """The same on tensors that are already stacked over the references: pres / feats = {layer: [B*R, ...]}, pairs laid
-        out [B, R] (what MRefSRPipeline.correspondences returns: no per-reference lists, no re-stacking)."""
-        for name, key in self._SCALES:
+        out [B, R] (what MRefSRPipeline.correspondences returns: no per-reference lists, no re-stacking).
+        pres may instead be the int64 arg-max map [B*R, h-2, w-2] at the 1/4-resolution grid
+        (correspondences(..., as_max_idx=True)): each DynAgg then runs forward_fused at its flow scale 1 / 2 / 4, whose
+        autograd node builds offsets and masks inside the DCN gather in the forward and in the backward."""
+        fused = torch.is_tensor(pres)
+        for s, (name, key) in zip((1, 2, 4), self._SCALES):
             conv1, conv2 = getattr(self, f'{name}_offset_conv1'), getattr(self, f'{name}_offset_conv2')
             agg = getattr(self, f'{name}_dyn_agg')
-            feat, pre = feats[key], pres[key]
+            feat = feats[key]
             feat_c = feat           # the DCN reads planes (NCHW); the convolution takes the trunk's layout
             if x.is_contiguous(memory_format=torch.channels_last) and not x.is_contiguous():
                 feat_c = feat.contiguous(memory_format=torch.channels_last)
@@ -217,13 +221,15 @@ class DynamicAggregationRestoration(nn.Module):
             o = self.lrelu(o)
             o2 = T.conv_bias_act_train(o, conv2, T.ACT_LEAKY, 0.1)
             o = o2 if o2 is not None else self.lrelu(conv2(o))
-            if agg.fused_autograd and T.layout_of(o) == 1:
+            if fused:
+                y = agg.forward_fused([feat, o], pres, s, out_slope=0.1, out_like_conv=True)  # [B*R, C, H, W]
+            elif agg.fused_autograd and T.layout_of(o) == 1:
                 # the leaky ReLU and the hand-off to the fusion head in the trunk's dtype / layout ride on the DynAgg
                 # node's one conversion pass (instead of an activation pass, then a cast (autocast) and a layout
                 # conversion (cuDNN) per convolution that reads the aligned features)
-                y = agg([feat, o], pre, out_slope=0.1, out_like_conv=True)                    # [B*R, C, H, W]
+                y = agg([feat, o], pres[key], out_slope=0.1, out_like_conv=True)              # [B*R, C, H, W]
             else:
-                y = self.lrelu(agg([feat, o], pre))
+                y = self.lrelu(agg([feat, o], pres[key]))
             h = getattr(self, f'head_{name}').forward_stacked(x, y, r)
             h = getattr(self, f'body_{name}')(h) + x
             tail = getattr(self, f'tail_{name}')
@@ -239,10 +245,12 @@ class DynamicAggregationRestoration(nn.Module):
 
     def forward(self, x, pre_offset_list, img_ref_feat_list, n_refs=None):
         """Reference contract: lists over references of pre_offset / VGG feature dicts.  Also accepted: the same tensors
-        already stacked over the references ({layer: [B*R, ...]} dicts, pairs laid out [B, R]) with n_refs = R."""
+        already stacked over the references ({layer: [B*R, ...]} dicts, pairs laid out [B, R]) with n_refs = R, where the
+        pre-offset dict may be replaced by the matcher's int64 arg-max map [B*R, h-2, w-2] (the fused DynAgg path)."""
         if isinstance(img_ref_feat_list, dict):
-            if n_refs is None or not isinstance(pre_offset_list, dict):
-                raise ValueError('stacked references: pass two {layer: [B*R, ...]} dicts and n_refs')
+            if n_refs is None or not (isinstance(pre_offset_list, dict) or torch.is_tensor(pre_offset_list)):
+                raise ValueError('stacked references: pass a {layer: [B*R, ...]} feature dict, a pre-offset dict or the '
+                                 'arg-max map, and n_refs')
             return self._forward_stacked(x, pre_offset_list, img_ref_feat_list, int(n_refs))
         if (self.batch_refs and len(img_ref_feat_list) > 1 and len(pre_offset_list) == len(img_ref_feat_list) and
                 all(f[k].shape == img_ref_feat_list[0][k].shape for f in img_ref_feat_list for _, k in self._SCALES)):
@@ -356,12 +364,14 @@ class MRefSRPipeline(nn.Module):
         return self.net_g.forward_batched(img_in_lq, max_idx, ref_feats, r)
 
     @torch.no_grad()
-    def correspondences(self, img_in_up, img_refs):
+    def correspondences(self, img_in_up, img_refs, as_max_idx=False):
         """The frozen half of a training step (MultiRefRestorationModel.optimize_parameters evaluates net_extractor and
         net_map per reference under no_grad, multi_ref_restoration_model.py:281-294 has the same loop for testing), batched
         over the references: one extractor pass over B*R reference images, ONE matcher launch for all pairs, one VGG pass.
         img_in_up [B,3,H,W], img_refs [B,R,3,H,W] -> (pre_offsets, ref_feats, R): {layer: [B*R, 9, s*h, s*w, 2]} and
-        {layer: [B*R, C, s*h, s*w]} with pairs laid out [B, R] -- the stacked form net_g.forward accepts."""
+        {layer: [B*R, C, s*h, s*w]} with pairs laid out [B, R] -- the stacked form net_g.forward accepts.
+        as_max_idx: return the matcher's int64 arg-max map [B*R, h-2, w-2] in place of the pre-offsets (no pre-offset
+        tensors are written; net_g then trains on the fused DynAgg path)."""
         b, r = img_refs.shape[:2]
         if self._channels_last:     # (channels_last_(): the frozen nets run cuDNN's NHWC kernels without layout conversions)
             img_in_up = img_in_up.contiguous(memory_format=torch.channels_last)
@@ -369,9 +379,9 @@ class MRefSRPipeline(nn.Module):
         f1, f2 = self.net_extractor.forward_batched(img_in_up, img_refs)
         idx, _ = feature_match_index_batched(f1, f2, 3, 1, 1, True, True, normalize_pixels=True, in_div=r,
                                              mode=self.match_mode)
-        o1, o2, o4 = pre_offsets(idx)
+        pres = idx if as_max_idx else dict(zip(('relu3_1', 'relu2_1', 'relu1_1'), pre_offsets(idx)))
         feats = self.net_map.vgg(img_refs.flatten(0, 1))
-        return {'relu3_1': o1, 'relu2_1': o2, 'relu1_1': o4}, {k: feats[k] for k in ('relu3_1', 'relu2_1', 'relu1_1')}, r
+        return pres, {k: feats[k] for k in ('relu3_1', 'relu2_1', 'relu1_1')}, r
 
     def forward_ragged(self, samples, max_batch=16, graphs=False):
         """Images with different reference counts / sizes (LMR-shaped groups, BASELINE config 3): samples[i] =

@@ -3,7 +3,7 @@ torchrun), 5 refs @160^2, through this repo's DynAgg / DCNv2 / MRAPAFusion autog
 boundaries: materialised pre-offsets, modulated_deform_conv backward for offset / mask / weight / bias, fusion
 backward).  The matcher has no backward (its only consumed output is the integer arg-max, SURVEY.md section 3.2).
 
-  python tools/train_step_bench.py [--batch 4] [--steps 5] [--bf16]
+  python tools/train_step_bench.py [--batch 4] [--steps 5] [--bf16] [--fused-dynagg]
   python -m torch.distributed.run --nproc-per-node N tools/train_step_bench.py ...
 Prints one JSON line on rank 0."""
 import argparse
@@ -26,7 +26,12 @@ ap.add_argument('--hr', type=int, default=160)
 ap.add_argument('--channels-last', action='store_true', help='run net_g in torch.channels_last (cuDNN native layout)')
 ap.add_argument('--per-reference', action='store_true', help='evaluate the frozen nets once per reference (the reference model structure)')
 ap.add_argument('--bf16', action='store_true', help='bf16 autocast for the plain convolutions (hot-path ops stay fp32)')
+ap.add_argument('--fused-dynagg', action='store_true',
+                help='train on the fused DynAgg path: correspondences(..., as_max_idx=True) -> net_g(lq, max_idx, feats, r), '
+                     'offsets / masks built inside the DCN gather in the forward and the backward')
 args = ap.parse_args()
+if args.fused_dynagg and args.per_reference:
+    ap.error('--fused-dynagg takes the batched correspondences (no --per-reference)')
 
 rank, world = int(os.environ.get('RANK', 0)), int(os.environ.get('WORLD_SIZE', 1))
 local = int(os.environ.get('LOCAL_RANK', 0))
@@ -72,7 +77,7 @@ def step():
                 rfs.append(rf)
         n_refs = None
     else:                       # the same, batched over the references (one extractor / matcher / VGG pass)
-        pres, rfs, n_refs = pipe.correspondences(up, refs_stacked)
+        pres, rfs, n_refs = pipe.correspondences(up, refs_stacked, as_max_idx=args.fused_dynagg)
     opt.zero_grad(set_to_none=True)
     x_in = lq.contiguous(memory_format=torch.channels_last) if args.channels_last else lq
     with torch.autocast('cuda', dtype=torch.bfloat16, enabled=args.bf16):
@@ -85,6 +90,7 @@ def step():
 
 losses = [float(step()) for _ in range(2)]
 torch.cuda.synchronize()
+torch.cuda.reset_peak_memory_stats(dev)
 if world > 1:
     dist.barrier()
 t0 = time.perf_counter()
@@ -97,7 +103,8 @@ if world > 1:
 grads_ok = all(p.grad is not None and torch.isfinite(p.grad).all() for p in net_g.parameters())
 if rank == 0:
     print(json.dumps({'test': 'train_step', 'n_gpus': world, 'batch_per_gpu': b, 'refs': r, 'hr': H, 'bf16_convs': args.bf16,
-                      'ms_per_step': float(dt) * 1e3, 'images_per_s': b * world / float(dt), 'losses': [round(x, 5) for x in losses],
+                      'fused_dynagg': args.fused_dynagg, 'ms_per_step': float(dt) * 1e3,
+                      'max_memory_allocated_gb': torch.cuda.max_memory_allocated(dev) / 2 ** 30, 'images_per_s': b * world / float(dt), 'losses': [round(x, 5) for x in losses],
                       'loss_decreasing': losses[-1] < losses[0], 'all_grads_finite': bool(grads_ok)}), flush=True)
 if world > 1:
     dist.destroy_process_group()
