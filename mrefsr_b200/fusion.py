@@ -62,11 +62,20 @@ class MRAPAAttentionFunction(Function):
 
 def mrapa_attention(emb_t, emb, ass, t):
     """emb_t [n,C,h,w] (already scaled by C**-0.5), emb [n*t,C,h,w], ass [n*t,Cv,h,w] -> [n,Cv,h,w].
-    Three bf16 tensors that need no gradient take the bf16-I/O kernel (`mrapa_attention_bf16`)."""
+    Three bf16 tensors that need no gradient take the bf16-I/O kernel (`mrapa_attention_bf16`) when it serves them;
+    the calls it refuses (more than 8 references, h*w % 4 != 0, planes not 8-byte aligned) run in fp32 and return bf16."""
     if (emb_t.dtype == emb.dtype == ass.dtype == torch.bfloat16 and
-            not (torch.is_grad_enabled() and (emb_t.requires_grad or emb.requires_grad or ass.requires_grad))):
+            not (torch.is_grad_enabled() and (emb_t.requires_grad or emb.requires_grad or ass.requires_grad)) and
+            _bf16_kernel_serves(emb_t, emb, ass, t)):
         return mrapa_attention_bf16(emb_t, emb, ass, t)
     return MRAPAAttentionFunction.apply(emb_t, emb, ass, t)
+
+
+def _bf16_kernel_serves(emb_t, emb, ass, t):
+    """What mrefsr_mrapa_attention_forward_bf16 accepts: t <= 8, h*w % 4 == 0 and 8-byte-aligned tensors.  A tensor
+    that is not contiguous is copied by mrapa_attention_bf16 into a fresh (aligned) allocation."""
+    return (t <= 8 and emb_t.dim() == 4 and emb_t.shape[2] * emb_t.shape[3] % 4 == 0 and
+            all(not x.is_contiguous() or x.data_ptr() % 8 == 0 for x in (emb_t, emb, ass)))
 
 
 def mrapa_attention_bf16(emb_t, emb, ass, t):
